@@ -243,5 +243,9 @@ def test_contrastive_mirrors_have_the_reference_surface(golden_contrastive):
             assert hasattr(lit, attr)
         cfg = lit.configure_optimizers()
         assert isinstance(cfg["optimizer"], torch.optim.Optimizer) and cfg["lr_scheduler"]["monitor"] == "train_loss"
-        with pytest.raises(Exception):                       # no CPU fallback
-            lit.training_step((torch.rand(2, 1, 28, 28), torch.rand(2, 1, 112, 112), torch.rand(2, 1, 28, 28), torch.rand(2, 1, 112, 112)), 0)
+        batch = (torch.rand(2, 1, 28, 28), torch.rand(2, 1, 112, 112), torch.rand(2, 1, 28, 28), torch.rand(2, 1, 112, 112))
+        if torch.cuda.is_available():                        # no CPU fallback: a host batch is stepped on the device
+            assert lit.training_step(batch, 0).is_cuda
+        else:
+            with pytest.raises(Exception):
+                lit.training_step(batch, 0)

@@ -122,11 +122,20 @@ def test_augment_survey_known_answer(golden):
 
 
 def test_affine_index_map_matches_torchvision():
-    """Bit-exact integer gather maps for NEAREST rotate/affine (SURVEY Appendix A1)."""
-    tv = pytest.importorskip("torchvision")
-    import torchvision.transforms.functional as F
-    from torchvision.transforms import InterpolationMode
+    """Bit-exact integer gather maps for NEAREST rotate/affine (SURVEY Appendix A1).  tests/golden/affine_torchvision.json holds
+    the SHA-256 of torchvision 0.26's map (int64, -1 = fill) for each case below, so the check needs no torchvision; where
+    torchvision is installed its maps are compared directly as well."""
+    import hashlib
+    import json
+    try:
+        import torchvision.transforms.functional as F
+        from torchvision.transforms import InterpolationMode
+    except ImportError:
+        F = None
+    with open(os.path.join(ROOT, "tests", "golden", "affine_torchvision.json")) as f:
+        digests = json.load(f)["sha256"]
     rng = np.random.default_rng(3)
+    i = 0
     for S in (28, 112):
         img = (torch.arange(S * S, dtype=torch.float32) + 1).view(1, S, S)
         for t in range(40):
@@ -134,13 +143,21 @@ def test_affine_index_map_matches_torchvision():
             tx, ty = int(rng.integers(-S // 5, S // 5 + 1)), int(rng.integers(-S // 5, S // 5 + 1))
             sc = float(rng.uniform(0.7, 1.3))
             if t % 2:
-                out = F.rotate(img, ang, interpolation=InterpolationMode.NEAREST, fill=[0.0])
                 m = AR.inverse_affine_matrix(-ang, 0, 0, 1.0)
             else:
-                out = F.affine(img, ang, [tx, ty], sc, [0.0, 0.0], interpolation=InterpolationMode.NEAREST, fill=[0.0])
                 m = AR.inverse_affine_matrix(ang, tx, ty, sc)
+            got = AR.affine_index_map(m, S, S).astype(np.int64)
+            assert hashlib.sha256(got.tobytes()).hexdigest() == digests[i], (S, t)
+            i += 1
+            if F is None:
+                continue
+            if t % 2:
+                out = F.rotate(img, ang, interpolation=InterpolationMode.NEAREST, fill=[0.0])
+            else:
+                out = F.affine(img, ang, [tx, ty], sc, [0.0, 0.0], interpolation=InterpolationMode.NEAREST, fill=[0.0])
             ref = out.numpy().reshape(S, S).astype(np.int64) - 1
-            assert np.array_equal(ref, AR.affine_index_map(m, S, S))
+            assert np.array_equal(ref, got)
+    assert i == len(digests)
 
 
 def _bias_cancelled_by_bn(name):
