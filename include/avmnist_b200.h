@@ -141,7 +141,8 @@ int b200_aug_apply_audio(const void* src, int src_u8, const int32_t* ops, const 
                          void* stream);
 /* device-side parameter sampling: spec tables int32 [4][B200_AUG_MAX_OPS][8] in the order
  * image-global, image-local, audio-global, audio-local (kind, p, a0..a5 as float bits; see augment.py pack_spec);
- * fills img_ops/aud_ops/group_bits for B samples x (Vg+Vl) views from Philox(seed, step). */
+ * fills img_ops/aud_ops/group_bits for B samples x (Vg+Vl) views from Philox(seed, step).  img_ops may be NULL (audio-only
+ * models): the image records are then neither drawn nor written, and the audio records and group bits are unchanged. */
 int b200_aug_sample(const int32_t* spec, int B, int Vg, int Vl, uint64_t seed, uint64_t step, int32_t* img_ops,
                     int32_t* aud_ops, uint32_t* group_bits, void* stream);
 /* CUDA-graph replay variants: the step counter lives in device memory (int64, advanced by b200_counters_advance inside the

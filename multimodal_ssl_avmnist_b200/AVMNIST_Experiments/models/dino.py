@@ -7,9 +7,10 @@ Adam -- runs in hand-written sm_100a kernels behind libavmnist_b200.so (multimod
 There is no PyTorch fallback: on a CPU tensor, or without the library, the step raises.
 
 Compiled encoders: CentralMultiModalEncoder ("multi_central"), the conv encoders SimpleMultiModalEncoder ("multi_simple"),
-GatedMultiModalEncoder ("multi_simple_gated") and CrossAttentionMultiModalEncoder ("multi_cross_attention") (SURVEY 8f-4), and
-ImageEncoder ("image_simple").  The other encoder families of the reference (LSTM, ViT, MobileViT, ResNet, spectrogram-only)
-are outside the hot-path scope; their names exist so that driver scripts import, and constructing one raises NotImplementedError.
+GatedMultiModalEncoder ("multi_simple_gated") and CrossAttentionMultiModalEncoder ("multi_cross_attention") (SURVEY 8f-4), and the
+unimodal ImageEncoder ("image_simple") and SpectrogramEncoder ("spectrogram_simple").  The other encoder families of the reference
+(LSTM, ViT, MobileViT, ResNet, the other spectrogram encoders) are outside the hot-path scope; their names exist so that driver
+scripts import, and constructing one raises NotImplementedError.
 """
 import os
 import sys
@@ -185,9 +186,10 @@ class ImageEncoder(BaseUniModalEncoder):
 
 
 class SpectrogramEncoder(BaseUniModalEncoder):
-    """audio_encoder(output_dim) on the spectrogram (reference models/dino.py:502-513).  Used by the stand-alone contrastive models
-    (other_ssl/info_nce, other_ssl/multimodal_simclr); as a unimodal DINO encoder it has no compiled step (B200_KIND None)."""
-    B200_KIND = None
+    """audio_encoder(output_dim) on the spectrogram (reference models/dino.py:502-513).  The audio-only DINO encoder
+    (UniModalDINO, `--unimodal_model spectrogram_simple`) and the audio branch of the stand-alone contrastive models
+    (other_ssl/info_nce, other_ssl/multimodal_simclr)."""
+    B200_KIND = "spectrogram_simple"
 
     def __init__(self, output_dim=256):
         super().__init__(output_dim, modality="audio")
@@ -202,7 +204,7 @@ class SpectrogramEncoder(BaseUniModalEncoder):
 def _out_of_scope(name):
     def __init__(self, *a, **k):
         raise NotImplementedError(f"{name} is outside the B200 hot-path scope (see DESIGN.md section 7); "
-                                  "compiled encoders: Central / Simple / Gated / CrossAttention MultiModalEncoder, ImageEncoder")
+                                  "compiled encoders: Central / Simple / Gated / CrossAttention MultiModalEncoder, ImageEncoder, SpectrogramEncoder")
     return type(name, (nn.Module,), {"__init__": __init__, "B200_KIND": None})
 
 
@@ -250,7 +252,7 @@ class _DinoBase(nn.Module):
         kind = getattr(encoder_class, "B200_KIND", None)
         if kind is None:
             raise NotImplementedError(f"{encoder_class.__name__} has no compiled B200 training step "
-                                      "(compiled: Central / Simple / Gated / CrossAttention MultiModalEncoder, ImageEncoder)")
+                                      "(compiled: Central / Simple / Gated / CrossAttention MultiModalEncoder, ImageEncoder, SpectrogramEncoder)")
         self._b200 = B.EngineBinding(self, kind, self.MODE)
         self.student_temperature, self.teacher_temperature = 0.1, 0.04
         self.n_global_views, self.n_local_views = 2, 4
@@ -377,14 +379,34 @@ class UniModalDINO(_DinoBase):
         self._setup(encoder_class, kw, output_dim, projection_dim, momentum, center_momentum, dropout)
 
     def forward(self, batch):
-        """Returns (student_outputs [V,B,P], teacher_outputs [Vg,B,P] (centred), embeddings [V,B,O])."""
+        """batch = (global_images, global_audios, local_images, local_audios) views; the encoder's modality is used ('image':
+        gi / li, 'audio': ga / la).  Returns (student_outputs [V,B,P], teacher_outputs [Vg,B,P] (centred), embeddings [V,B,O])."""
         gi, ga, li, la = self._views(batch)
-        if self.student.modality != "image":
-            raise NotImplementedError("only the image modality has a compiled unimodal step")
-        out = self._b200.forward(_to_view_major(gi, li), None)
-        w = self._b200.last_w
-        emb = w["s.feat"].view(gi.shape[1] + li.shape[1], gi.shape[0], -1)
-        return out[0], out[1], emb
+        if self.student.modality == "image":
+            out = self._b200.forward(_to_view_major(gi, li), None)
+        else:
+            out = self._b200.forward(None, _to_view_major(ga, la))
+        return out[0], out[1], self._embeddings(gi.shape[0])
+
+    def _embeddings(self, B):
+        eng = self.engine
+        return self._b200.last_w["s.feat"].view(eng.V, B, -1)
+
+    def forward_raw(self, images, audios, augment_values="keep"):
+        """B200 fast path: un-augmented device batch (images [B,1,28,28] fp32/uint8, audios [B,1,112,112] uint8/fp32; the
+        modality the encoder does not read may be None) -> device-sampled multi-crop augmentation of the encoder's modality, written
+        straight into the first convolution's operand format -> the same outputs as forward()."""
+        dev = self.center.device
+        eng = self._b200.ensure(dev)
+        if augment_values != "keep":
+            eng.set_augmentation(augment_values)
+        if self.student.modality == "image":
+            img, aud = images.to(dev).reshape(-1, 28, 28).contiguous(), None
+        else:
+            img, aud = None, audios.to(dev).reshape(-1, 112, 112).contiguous()
+        xi, xa = eng.augment(img, aud, direct=True)
+        out = self._b200.forward(xi, xa)
+        return out[0], out[1], self._embeddings((img if img is not None else aud).shape[0])
 
 
 # ------------------------------------------------------------------------------------------------------------
@@ -412,8 +434,13 @@ class FeatureExtractor(nn.Module):
         eng = dino._b200.ensure(dino.center.device)
         if self._probe is None:
             self._probe = eng.begin_probe()
-        img = images.to(eng.device).reshape(-1, 28, 28).contiguous()
-        aud = None if (self.is_unimodal or spectrograms is None) else spectrograms.to(eng.device).reshape(-1, 112, 112).contiguous()
+        img = aud = None
+        if self.modality != "audio":
+            img = images.to(eng.device).reshape(-1, 28, 28).contiguous()
+        if self.modality == "audio" or not (self.is_unimodal or spectrograms is None):
+            if spectrograms is None:
+                raise ValueError("an audio-only model needs the spectrograms")
+            aud = spectrograms.to(eng.device).reshape(-1, 112, 112).contiguous()
         return eng.encode_features(img, aud, train=self.training, probe=self._probe).clone()
 
 
@@ -452,6 +479,11 @@ class _DinoLightningBase(pl.LightningModule):
 
     def forward(self, batch):
         return self.model(batch)
+
+    def _augment_values(self):
+        dm = getattr(getattr(self, "trainer", None), "datamodule", None)
+        aug = getattr(dm, "augmentations", None)
+        return getattr(aug, "augment_values", None)
 
     def dino_loss(self, student_outputs, teacher_outputs, alignment_loss=None):
         """Centred, temperature-sharpened cross-entropy over all student x teacher view pairs (fused CUDA kernel)."""
@@ -543,11 +575,6 @@ class MultiModalDINOLightning(_DinoLightningBase):
                                       encoder_output_dim=self.encoder_output_dim, projection_dim=self.projection_dim,
                                       momentum=self.momentum, center_momentum=self.center_momentum, dropout=self.dropout)
         return self.model
-
-    def _augment_values(self):
-        dm = getattr(getattr(self, "trainer", None), "datamodule", None)
-        aug = getattr(dm, "augmentations", None)
-        return getattr(aug, "augment_values", None)
 
     def training_step(self, batch, batch_idx):
         self._sync_hparams()
@@ -669,8 +696,25 @@ class UniModalDINOLightning(_DinoLightningBase):
         return B.standalone_cosine_loss(embeddings)
 
     def training_step(self, batch, batch_idx):
+        """batch = the reference's 4-tuple of views, or a raw (image, audio[, label]) batch that is augmented on the device (the
+        default AVMNISTDinoDataModule); small raw batches take the fused CUDA-graph step like the multimodal modules."""
         self._sync_hparams()
-        student_out, teacher_out, embeddings = self.model(batch)
+        if len(batch) in (2, 3) and batch[0].dim() == 4:          # raw (image, audio[, label]) batch: augment on the device
+            av = "keep" if getattr(self, "_aug_set", False) else self._augment_values()
+            self._aug_set = True
+            audio_only = self.model.student.modality == "audio"
+            if self._use_fused_step(batch[0].shape[0]):           # small batch: the whole step is one CUDA-graph replay
+                dev = self.model.center.device
+                if av != "keep":
+                    self.model._b200.ensure(dev).set_augmentation(av)
+                images, audios = (None, batch[1].to(dev)) if audio_only else (batch[0].to(dev), None)
+                loss = self.model._b200.fused_train_step(images, audios, cosine_loss_alpha=float(self.cosine_loss_alpha))
+                if loss is not None:
+                    self.log("train_loss", loss, on_step=True, on_epoch=True, prog_bar=True)
+                    return loss
+            student_out, teacher_out, embeddings = self.model.forward_raw(None if audio_only else batch[0], batch[1] if audio_only else None, av)
+        else:
+            student_out, teacher_out, embeddings = self.model(batch)
         loss = self.dino_loss(student_out, teacher_out)
         cosine_loss = None
         if self.cosine_loss_alpha > 0:

@@ -225,10 +225,11 @@ class EngineBinding:
 
     # ---- the step, as autograd-visible pieces ------------------------------------------------------------------
     def forward(self, x_img, x_aud, raw=None, masks=None):
-        """x_img [V,B,28,28] / x_aud [V,B,112,112] view-major device tensors.  Returns (student_out [V,B,P], teacher_out
-        [Vg,B,P] centred with the pre-update centre[, image_out, audio_out])."""
-        eng = self.ensure(x_img.device)
-        B = x_img.shape[1]
+        """x_img [V,B,28,28] / x_aud [V,B,112,112] view-major device tensors (None for a modality the kind does not encode).
+        Returns (student_out [V,B,P], teacher_out [Vg,B,P] centred with the pre-update centre[, image_out, audio_out])."""
+        x_in = x_img if x_img is not None else x_aud
+        eng = self.ensure(x_in.device)
+        B = x_in.shape[1]
         center_before = eng.center.clone()
         w = eng.forward_pass(x_img, x_aud, masks=masks, raw=raw)
         eng.dino_loss_pass(w)             # fused loss fwd+bwd + centre EMA (the reference updates the centre inside forward)
@@ -244,29 +245,36 @@ class EngineBinding:
         eng.rng_step += 1
         return (res[0], teacher_c) + tuple(res[1:])
 
-    def fused_train_step(self, images, audios, labels=None, alpha=1.0):
+    def fused_train_step(self, images, audios, labels=None, alpha=1.0, cosine_loss_alpha=None):
         """The WHOLE training step of a raw device batch as one CUDA-graph replay (augmentation, forward, losses, centre / teacher EMA,
         backward, gradient exchange, Adam): for small per-GPU batches, where the ~165 launches of the step-by-step module path cost
         more host time than GPU time (B = 128: 3.0 -> 1.9 ms).  The graph is captured on first use per batch size; the learning rate
         follows the optimizer's param_groups (device scalar), Adam state belongs to the current B200Adam.  Returns the total loss as
         an autograd-visible scalar whose backward is a no-op, and marks the step as applied for the next optimizer.step(); None if a
-        graph for a different batch size / weight decay / alpha is already captured (the caller then takes the step-by-step path)."""
-        eng = self.ensure(images.device)
+        graph for a different batch size / weight decay / alpha is already captured (the caller then takes the step-by-step path).
+        images or audios may be None for a modality the kind does not encode; cosine_loss_alpha (unimodal kinds) sets the weight of
+        the cosine-consistency term baked into the graph (None: the engine's current value)."""
+        x_in = images if images is not None else audios
+        eng = self.ensure(x_in.device)
         opt = self.optimizer
         if opt is None:
             raise ops._lib.B200Error("fused_train_step needs the B200Adam from configure_optimizers()")
         opt._claim_engine(eng)
         g0 = opt.param_groups[0]
         eng.lr = g0["lr"]
-        img = images.reshape(-1, 28, 28).contiguous()
+        img = None if images is None else images.reshape(-1, 28, 28).contiguous()
         aud = None if audios is None else audios.reshape(-1, 112, 112).contiguous()
-        B = img.shape[0]
-        key = (B, img.dtype, None if aud is None else aud.dtype, float(g0["weight_decay"]), float(alpha))
+        B = (img if img is not None else aud).shape[0]
+        cos = float(eng.cosine_loss_alpha if cosine_loss_alpha is None else cosine_loss_alpha)
+        key = (B, None if img is None else img.dtype, None if aud is None else aud.dtype, float(g0["weight_decay"]), float(alpha))
+        if cos != 0.0:
+            key += (cos,)
         if eng._graph is not None and eng._graph.get("key") != key:
             return None                    # a graph for another batch size / setting exists: this batch takes the step-by-step path
         if eng._graph is None:
-            eng.weight_decay, eng.alpha = g0["weight_decay"], float(alpha)
-            eng.capture_train_step(B, image_dtype=img.dtype, audio_dtype=torch.uint8 if aud is None else aud.dtype)
+            eng.weight_decay, eng.alpha, eng.cosine_loss_alpha = g0["weight_decay"], float(alpha), cos
+            eng.capture_train_step(B, image_dtype=torch.float32 if img is None else img.dtype,
+                                   audio_dtype=torch.uint8 if aud is None else aud.dtype)
             eng._graph["key"] = key
         loss = eng.graph_step(img, aud, labels)
         self.step_applied = True

@@ -554,7 +554,9 @@ __global__ void __launch_bounds__(32 * SAMPLE_WARPS) aug_sample_kernel(const int
     int gc = -1;
     if (tid == 0) {
         Draw di(seed, stream | 2), da(seed, stream | 3);
-        sample_chain(sspec + (local ? 1 : 0) * B200_AUG_MAX_OPS * 8, 28, di, rec_i, &gc);
+        // the two chains draw from separate streams and only the audio chain sets gc: skipping the image records (img_ops NULL,
+        // audio-only models) leaves the audio records and the group mask unchanged
+        if (img_ops != nullptr) sample_chain(sspec + (local ? 1 : 0) * B200_AUG_MAX_OPS * 8, 28, di, rec_i, &gc);
         sample_chain(sspec + (local ? 3 : 2) * B200_AUG_MAX_OPS * 8, 112, da, rec_a, &gc);
         if (gc > NGROUPS) gc = NGROUPS;
     }
@@ -617,7 +619,7 @@ __global__ void __launch_bounds__(32 * SAMPLE_WARPS) aug_sample_kernel(const int
     }
     __syncwarp();
     for (int i = tid; i < B200_AUG_MAX_OPS * 8; i += 32) {
-        img_ops[rec * (B200_AUG_MAX_OPS * 8) + i] = rec_i[i];
+        if (img_ops != nullptr) img_ops[rec * (B200_AUG_MAX_OPS * 8) + i] = rec_i[i];
         aud_ops[rec * (B200_AUG_MAX_OPS * 8) + i] = rec_a[i];
     }
     if (tid < B200_AUG_GROUP_WORDS) group_bits[rec * B200_AUG_GROUP_WORDS + tid] = bits[tid];
@@ -673,7 +675,7 @@ int b200_aug_sample(const int32_t* spec, int B, int Vg, int Vl, uint64_t seed, u
 
 int b200_aug_sample_dev(const int32_t* spec, int B, int Vg, int Vl, uint64_t seed, uint64_t step, const int64_t* step_dev, int32_t* img_ops,
                         int32_t* aud_ops, uint32_t* group_bits, void* stream) {
-    B200_REQUIRE(spec && img_ops && aud_ops && group_bits && B > 0 && Vg >= 0 && Vl >= 0 && Vg + Vl > 0, B200_E_ARG,
+    B200_REQUIRE(spec && aud_ops && group_bits && B > 0 && Vg >= 0 && Vl >= 0 && Vg + Vl > 0, B200_E_ARG,
                  "aug_sample: bad arguments");
     const long recs = (long)B * (Vg + Vl);
     aug_sample_kernel<<<(unsigned)((recs + SAMPLE_WARPS - 1) / SAMPLE_WARPS), 32 * SAMPLE_WARPS, 0, as_stream(stream)>>>(spec, B, Vg, Vl, seed, step, img_ops,

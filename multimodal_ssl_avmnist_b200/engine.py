@@ -14,7 +14,8 @@ streams; for data parallel runs the two exchanges (gradient arena, centre column
 
 Encoders (`kind`): 'multi_central' (CentralMultiModalEncoder, the headline), 'multi_simple' / 'multi_simple_gated' /
 'multi_cross_attention' (the 3x3 conv encoders of models/dino.py:214-263, 385-452: stack tops are avgpool -> linear and a mix stage --
-sigmoid gates or batch-wide cross attention -- sits before the fusion MLP) and 'image_simple' (unimodal).  The stand-alone contrastive
+sigmoid gates or batch-wide cross attention -- sits before the fusion MLP), and the unimodal 'image_simple' (ImageEncoder) and
+'spectrogram_simple' (SpectrogramEncoder: the audio stack of 'multi_simple' alone).  The stand-alone contrastive
 steps of other_ssl/ reuse these building blocks from contrastive.ContrastiveStepEngine.
 
 Arena layout (student):  [ encoder params that receive gradients | projection head | unused fc1/fc2 | mode heads ]
@@ -89,6 +90,15 @@ def image_simple_params(O):
     return used, []
 
 
+def spectrogram_simple_params(O):
+    """SpectrogramEncoder (models/dino.py:502-513) = audio_encoder(O): four conv blocks and Linear(256, O), no projection layer."""
+    used = []
+    for i, (ci, co) in zip((0, 4, 8, 12), ((1, 32), (32, 64), (64, 128), (128, 256))):
+        used += _conv(f"encoder.{i}", co, ci, 3) + _vec2(f"encoder.{i + 1}", co)
+    used += _lin("encoder.18", O, 256)
+    return used, []
+
+
 def simple_multi_params(E, O, mix=None):
     """Parameter specs of SimpleMultiModalEncoder (models/dino.py:214-234: image_encoder() / audio_encoder() `nn.Sequential`s,
     :18-73, + the concatenation fusion) and its two subclasses: GatedMultiModalEncoder (:237-263, two scalar gates) and
@@ -125,8 +135,14 @@ MULTI_SIMPLE_IMAGE_LAYERS = [("image_encoder.0", "image_encoder.1", 1, 32, 28, 3
                              ("image_encoder.8", "image_encoder.9", 64, 128, 7, 3, 1)]
 MULTI_SIMPLE_AUDIO_LAYERS = [("audio_encoder.0", "audio_encoder.1", 1, 32, 112, 3, 1), ("audio_encoder.4", "audio_encoder.5", 32, 64, 56, 3, 1),
                              ("audio_encoder.8", "audio_encoder.9", 64, 128, 28, 3, 1), ("audio_encoder.12", "audio_encoder.13", 128, 256, 14, 3, 1)]
+SPECTROGRAM_LAYERS = [("encoder.0", "encoder.1", 1, 32, 112, 3, 1), ("encoder.4", "encoder.5", 32, 64, 56, 3, 1),
+                      ("encoder.8", "encoder.9", 64, 128, 28, 3, 1), ("encoder.12", "encoder.13", 128, 256, 14, 3, 1)]
 # kind -> feature mixing between the encoders and the fusion MLP
 MULTI_KINDS = {"multi_central": None, "multi_simple": None, "multi_simple_gated": "gated", "multi_cross_attention": "cross"}
+# unimodal kind -> (modality stack, width of the global average pool, [(linear, input buffer, output buffer, output width)] after the
+# pool; the last output is the embedding `feat` that the projection head and the cosine-consistency term read)
+UNI_KINDS = {"image_simple": ("img", 128, [("enc.encoder.14", "pool", "e14", 512), ("enc.projection.0", "e14", "feat", None)]),
+             "spectrogram_simple": ("aud", 256, [("enc.encoder.18", "pool", "feat", None)])}
 
 
 class Arena:
@@ -166,6 +182,11 @@ class _BN:
         self.num_batches_tracked = torch.zeros(1, dtype=torch.int64, device=device)
 
 
+def _rows(x, n):
+    """The first n rows of an optional input buffer."""
+    return None if x is None else x[:n]
+
+
 def _main_chain(fn):
     """Method decorator: the launches of `fn` go to the engine's high-priority main stream (DinoStepEngine._on_main)."""
     import functools
@@ -179,8 +200,10 @@ def _main_chain(fn):
 
 class DinoStepEngine:
     """See module docstring.  kind: 'multi_central' (CentralMultiModalEncoder), 'multi_simple' (SimpleMultiModalEncoder),
-    'multi_simple_gated' (GatedMultiModalEncoder), 'multi_cross_attention' (CrossAttentionMultiModalEncoder) or 'image_simple'
-    (ImageEncoder); mode: 'default' | 'semi_supervised' | 'infonce' | 'mse' (multimodal kinds only)."""
+    'multi_simple_gated' (GatedMultiModalEncoder), 'multi_cross_attention' (CrossAttentionMultiModalEncoder), 'image_simple'
+    (ImageEncoder) or 'spectrogram_simple' (SpectrogramEncoder); mode: 'default' | 'semi_supervised' | 'infonce' | 'mse' (multimodal
+    kinds only).  The unimodal kinds have one conv stack; the methods that take (images, audios) ignore the absent modality's
+    argument (it may be None) and allocate nothing for it."""
 
     def __init__(self, kind="multi_central", mode="default", encoder_output_dim=256, output_dim=256, projection_dim=128,
                  n_global_views=2, n_local_views=4, momentum=0.996, center_momentum=0.9, student_temperature=0.1,
@@ -191,7 +214,7 @@ class DinoStepEngine:
             raise ops._lib.B200Error("DinoStepEngine needs a CUDA device: the hot path has no CPU fallback")
         ops._lib.load()
         self.device = torch.device(device if device is not None else f"cuda:{torch.cuda.current_device()}")
-        assert kind in MULTI_KINDS or kind == "image_simple"
+        assert kind in MULTI_KINDS or kind in UNI_KINDS
         self.multi = kind in MULTI_KINDS
         self.mix = MULTI_KINDS.get(kind)
         assert mode == "default" or self.multi
@@ -227,10 +250,16 @@ class DinoStepEngine:
             used, unused = simple_multi_params(self.E, self.O, self.mix)
             self.img_layers, self.aud_layers = MULTI_SIMPLE_IMAGE_LAYERS, MULTI_SIMPLE_AUDIO_LAYERS
             self.top = {"img": (True, 128, "enc.image_encoder.14"), "aud": (True, 256, "enc.audio_encoder.18")}
-        else:
+        elif kind == "image_simple":
             used, unused = image_simple_params(self.O)
             self.img_layers, self.aud_layers = SIMPLE_IMAGE_LAYERS, []
             self.top = {}
+        else:
+            used, unused = spectrogram_simple_params(self.O)
+            self.img_layers, self.aud_layers = [], SPECTROGRAM_LAYERS
+            self.top = {}
+        # unimodal kinds: the modality of the one conv stack and the layers between its global average pool and the embedding
+        self.uni = UNI_KINDS.get(kind)
         head = [("head." + n, s) for n, s in head_params(self.O, self.P)]
         enc_used = [("enc." + n, s) for n, s in used]
         enc_unused = [("enc." + n, s) for n, s in unused]
@@ -440,13 +469,16 @@ class DinoStepEngine:
             return zarena[o:o + n].view(*shape)
 
         w["zarena"] = zarena
-        # augmentation
-        w["img_ops"] = torch.zeros(B, V, A.MAX_OPS, A.OP_WORDS, dtype=torch.int32, device=dev)
+        # augmentation (the sampler always draws the audio records; the image records only when there is an image stack)
+        if self.img_layers:
+            w["img_ops"] = torch.zeros(B, V, A.MAX_OPS, A.OP_WORDS, dtype=torch.int32, device=dev)
         w["aud_ops"] = torch.zeros(B, V, A.MAX_OPS, A.OP_WORDS, dtype=torch.int32, device=dev)
         w["group_bits"] = torch.zeros(B, V, A.GROUP_WORDS, dtype=torch.int32, device=dev)
         for nm in ("img_ops", "aud_ops", "group_bits"):
-            w[nm + "_b"] = torch.zeros_like(w[nm])
-        w["x_img"] = e(Ns, 1, 28, 28)
+            if nm in w:
+                w[nm + "_b"] = torch.zeros_like(w[nm])
+        if self.img_layers:
+            w["x_img"] = e(Ns, 1, 28, 28)
         if self.aud_layers:
             w["x_aud"] = e(Ns, 1, 112, 112)
         scr = {m: dict(wg=0, z=0, p=0, z8=0) for m in ("img", "aud")}       # backward scratch sizes per modality stack
@@ -527,10 +559,8 @@ class DinoStepEngine:
                         w[f"att{mi}.{nm}"] = e(Nv, E)
         else:
             for role, N in (("s", Ns), ("t", Nt)):
-                w[f"{role}.pool"] = e(N, 128)
-                w[f"{role}.e14"] = e(N, 512)
-                w[f"{role}.feat"] = e(N, O)
-            w["d.pool"], w["d.e14"] = e(Ns, 128), e(Ns, 512)
+                self._uni_workspace(w, role, N, e)
+            self._uni_workspace(w, "d", Ns, e, with_feat=False)
         w["d.feat"] = e(Nv, O)
         for role, N in (("s", Nv), ("t", Nt)):
             w[f"{role}.hh"] = e(N, 512)
@@ -563,6 +593,14 @@ class DinoStepEngine:
             w["d.emb"] = e(Nv, O)          # cosine-consistency gradient (UniModalDINO, cosine_loss_alpha may be switched on later)
         self._ws[B] = w
         return w
+
+    def _uni_workspace(self, w, role, N, e, with_feat=True):
+        """Unimodal kinds: the pooled features [N, pool width] and the outputs of the linears after the pool (`feat` [N, O] last)."""
+        _, width, chain = self.uni
+        w[f"{role}.pool"] = e(N, width)
+        for lin, src, dst, cols in chain:
+            if dst != "feat" or with_feat:
+                w[f"{role}.{dst}"] = e(N, self.O if cols is None else cols)
 
     def _mix_workspace(self, w, role, N, nfus, B, e):
         """Encoder-feature buffers of one role: catr [N, 2E] = (image | audio) features as the encoders' linears produce them, cat =
@@ -647,56 +685,75 @@ class DinoStepEngine:
     # ------------------------------------------------------------------------------------------------------
     # augmentation
     # ------------------------------------------------------------------------------------------------------
+    def _batch_size(self, images, audios):
+        """B of a raw batch, read from the modality the kind encodes first (the image batch, or the audio batch of an audio-only kind)."""
+        x = images if self.img_layers else audios
+        if x is None:
+            raise ops._lib.B200Error(f"{self.kind}: the {'image' if self.img_layers else 'audio'} batch is required")
+        return x.shape[0]
+
+    def _direct_views(self):
+        """Can the augmentation write the first-layer quad8 operands directly?  (Every stack's first layer is a tensor-core layer.)"""
+        return all(self.tc[m][0] for m, layers in (("img", self.img_layers), ("aud", self.aud_layers)) if layers)
+
     def prefetch_augment(self, images, audios):
         """Enqueue the NEXT step's sampling + augmentation on the augmentation stream, into the spare first-layer buffers, so
         that it overlaps the tail of the current step (its last weight gradient, EMA, Adam).  The next train_step() on the
         same tensors picks the views up instead of augmenting again.  Tensor-core path only; a no-op otherwise."""
-        if not (self.tc["img"][0] and (not self.aud_layers or self.tc["aud"][0])):
+        if not self._direct_views():
             return False
-        B = images.shape[0]
+        B = self._batch_size(images, audios)
         w = self._workspace(B)
         main, st = torch.cuda.current_stream(), self._aug_stream
         if self._step_done_prev is not None:
             st.wait_event(self._step_done_prev)       # the spare slot was last read by the step BEFORE the one in flight
         with torch.cuda.stream(st):
-            ops.aug_sample(self.aug_spec, B, self.Vg, self.Vl, self.seed, self.rng_step, w["img_ops_b"], w["aud_ops_b"], w["group_bits_b"])
+            ops.aug_sample(self.aug_spec, B, self.Vg, self.Vl, self.seed, self.rng_step, w.get("img_ops_b"), w["aud_ops_b"], w["group_bits_b"])
             seed = (self.seed * 1000003 + self.rng_step) & 0xFFFFFFFFFFFF
             V = self.V
-            pi = self.img_layers[0][6]
-            ops.aug_apply_image(images.reshape(B, 28, 28), w["img_ops_b"], None, out8=w["img.xs8_b"][:V * B].view(V, B, 28, ops.quad8_width(28, pi), 8), pad=pi)
+            if self.img_layers:
+                pi = self.img_layers[0][6]
+                ops.aug_apply_image(images.reshape(B, 28, 28), w["img_ops_b"], None, out8=w["img.xs8_b"][:V * B].view(V, B, 28, ops.quad8_width(28, pi), 8),
+                                    pad=pi)
             if self.aud_layers and audios is not None:
                 pa = self.aud_layers[0][6]
                 ops.aug_apply_audio(audios.reshape(B, 112, 112), w["aud_ops_b"], w["group_bits_b"], None, seed=seed,
                                     out8=w["aud.xs8_b"][:V * B].view(V, B, 112, ops.quad8_width(112, pa), 8), pad=pa)
             ev = torch.cuda.Event()
             ev.record(st)
-        self._prefetch = {"key": (images.data_ptr(), None if audios is None else audios.data_ptr(), B, self.rng_step), "event": ev}
+        self._prefetch = {"key": self._batch_key(images, audios), "event": ev}
         return True
+
+    def _batch_key(self, images, audios):
+        img = images if self.img_layers else None            # an audio-only kind ignores the image batch
+        return (None if img is None else img.data_ptr(), None if audios is None else audios.data_ptr(), self._batch_size(images, audios),
+                self.rng_step)
 
     def _take_prefetched(self, images, audios):
         """If the views of this batch were prefetched for this rng position: swap the buffer slots and return them."""
         pf, self._prefetch = self._prefetch, None
-        B = images.shape[0]
-        if pf is None or pf["key"] != (images.data_ptr(), None if audios is None else audios.data_ptr(), B, self.rng_step):
+        if pf is None or pf["key"] != self._batch_key(images, audios):
             return None
+        B = self._batch_size(images, audios)
         w = self._workspace(B)
         torch.cuda.current_stream().wait_event(pf["event"])
         for nm in ("img.xs8", "aud.xs8", "img_ops", "aud_ops", "group_bits"):
             if nm in w:
                 w[nm], w[nm + "_b"] = w[nm + "_b"], w[nm]
         V = self.V
-        xi = w["img.xs8"][:V * B].view(V, B, 28, ops.quad8_width(28, self.img_layers[0][6]), 8)
+        xi = w["img.xs8"][:V * B].view(V, B, 28, ops.quad8_width(28, self.img_layers[0][6]), 8) if self.img_layers else None
         xa = w["aud.xs8"][:V * B].view(V, B, 112, ops.quad8_width(112, self.aud_layers[0][6]), 8) if self.aud_layers else None
         return xi, xa
 
     def augment(self, images, audios, B=None, direct=False):
         """Device-sampled multi-crop views of a raw batch: images [B,28,28] (fp32 in [0,1] or uint8),
-        audios [B,112,112] (uint8 or fp32).  Returns view-major tensors ([V,B,28,28], [V,B,112,112])."""
-        B = images.shape[0]
+        audios [B,112,112] (uint8 or fp32).  Returns view-major tensors ([V,B,28,28], [V,B,112,112]); None for a modality the
+        kind does not encode."""
+        B = self._batch_size(images, audios)
         w = self._workspace(B)
         step, step_dev = self._step_args()
-        ops.aug_sample(self.aug_spec, B, self.Vg, self.Vl, self.seed, step, w["img_ops"], w["aud_ops"], w["group_bits"], step_dev=step_dev)
-        return self.augment_with_params(images, audios, w["img_ops"], w["aud_ops"], w["group_bits"], None, direct=direct)
+        ops.aug_sample(self.aug_spec, B, self.Vg, self.Vl, self.seed, step, w.get("img_ops"), w["aud_ops"], w["group_bits"], step_dev=step_dev)
+        return self.augment_with_params(images, audios, w.get("img_ops"), w["aud_ops"], w["group_bits"], None, direct=direct)
 
     def _step_args(self):
         """(host step value, device step counter) for the kernels that consume the RNG stream position: eager mode passes the
@@ -707,25 +764,27 @@ class DinoStepEngine:
         """Applies the op records.  direct=False: fp32 views ([V,B,28,28], [V,B,112,112]).  direct=True (tensor-core path
         only): the kernels write the first-layer quad8 images straight into the workspace (no fp32 round trip); the
         returned bf16 tensors are those workspace buffers and are recognised by forward_pass."""
-        B = images.shape[0]
+        B = self._batch_size(images, audios)
         w = self._workspace(B)
         V = self.V
         step, step_dev = self._step_args()
         seed = (self.seed * 1000003 + step) & 0xFFFFFFFFFFFF
-        if direct and self.tc["img"][0] and (not self.aud_layers or self.tc["aud"][0]):
-            pi = self.img_layers[0][6]
-            xi = w["img.xs8"][:V * B].view(V, B, 28, ops.quad8_width(28, pi), 8)
-            ops.aug_apply_image(images.reshape(B, 28, 28), img_ops, None, out8=xi, pad=pi)
-            xa = None
+        if direct and self._direct_views():
+            xi = xa = None
+            if self.img_layers:
+                pi = self.img_layers[0][6]
+                xi = w["img.xs8"][:V * B].view(V, B, 28, ops.quad8_width(28, pi), 8)
+                ops.aug_apply_image(images.reshape(B, 28, 28), img_ops, None, out8=xi, pad=pi)
             if self.aud_layers and audios is not None:
                 pa = self.aud_layers[0][6]
                 xa = w["aud.xs8"][:V * B].view(V, B, 112, ops.quad8_width(112, pa), 8)
                 ops.aug_apply_audio(audios.reshape(B, 112, 112), aud_ops, group_bits, None, noise=noise, seed=seed, out8=xa, pad=pa,
                                     step_dev=step_dev)
             return xi, xa
-        xi = w["x_img"][:V * B].view(V, B, 28, 28)
-        ops.aug_apply_image(images.reshape(B, 28, 28), img_ops, xi)
-        xa = None
+        xi = xa = None
+        if self.img_layers:
+            xi = w["x_img"][:V * B].view(V, B, 28, 28)
+            ops.aug_apply_image(images.reshape(B, 28, 28), img_ops, xi)
         if self.aud_layers and audios is not None:
             xa = w["x_aud"][:V * B].view(V, B, 112, 112)
             ops.aug_apply_audio(audios.reshape(B, 112, 112), aud_ops, group_bits, xa, noise=noise, seed=seed, step_dev=step_dev)
@@ -872,11 +931,16 @@ class DinoStepEngine:
                 ops.linear_fwd(cat[:n_fusion], P["enc.fusion.0.weight"], P["enc.fusion.0.bias"], h1, act=2, mask=fmask, drop_p=self.fusion_dropout, tc=self.lin_tc)
             ops.linear_fwd(h1, P["enc.fusion.3.weight"], P["enc.fusion.3.bias"], feat, tc=self.lin_tc)
             return feat
-        pi = self._conv_stack(w, role, "img", self.img_layers, x_img, N, B, P, bns, train=train)      # [N,128,3,3]
-        ops.avgpool_fwd(pi, w[f"{role}.pool"])
-        ops.linear_fwd(w[f"{role}.pool"], P["enc.encoder.14.weight"], P["enc.encoder.14.bias"], w[f"{role}.e14"], tc=self.lin_tc)
-        ops.linear_fwd(w[f"{role}.e14"], P["enc.projection.0.weight"], P["enc.projection.0.bias"], w[f"{role}.feat"], tc=self.lin_tc)
+        # unimodal: conv stack -> global average pool -> the linears of self.uni (image: encoder.14, projection.0; audio: encoder.18)
+        mod, _, chain = self.uni
+        p_last = self._conv_stack(w, role, mod, self._layers(mod), x_img if mod == "img" else x_aud, N, B, P, bns, train=train)
+        ops.avgpool_fwd(p_last, w[f"{role}.pool"])
+        for lin, src, dst, _ in chain:
+            ops.linear_fwd(w[f"{role}.{src}"], P[lin + ".weight"], P[lin + ".bias"], w[f"{role}.{dst}"], tc=self.lin_tc)
         return w[f"{role}.feat"]
+
+    def _layers(self, mod):
+        return self.img_layers if mod == "img" else self.aud_layers
 
     def _conv_stack_bwd(self, w, mod, layers, x, d_top, N, B):
         """Backward through a conv stack; d_top = gradient w.r.t. the last pooled activation (fp32, any shape, N*C*h*w)."""
@@ -985,7 +1049,8 @@ class DinoStepEngine:
         def e(*shape, dtype=F32):
             return torch.empty(*shape, dtype=dtype, device=dev)
 
-        w["x_img"] = e(B, 1, 28, 28)
+        if self.img_layers:
+            w["x_img"] = e(B, 1, 28, 28)
         if self.aud_layers:
             w["x_aud"] = e(B, 1, 112, 112)
         for mod, layers in (("img", self.img_layers), ("aud", self.aud_layers)):
@@ -1015,7 +1080,7 @@ class DinoStepEngine:
                 if self.top[mod][0]:
                     w[f"e.{mod}.gap"] = e(B, self.top[mod][1])
         else:
-            w["e.pool"], w["e.e14"], w["e.feat"] = e(B, 128), e(B, 512), e(B, O)
+            self._uni_workspace(w, "e", B, e)
         self._ws[key] = w
         return w
 
@@ -1042,7 +1107,7 @@ class DinoStepEngine:
         train=False: BatchNorm with running statistics, no dropout (module.eval()); train=True: batch statistics and an active
         fusion dropout.  probe (a begin_probe() token): the running statistics read / updated are the probe copy's, and every
         train-mode call draws a fresh dropout mask; without a token train-mode updates go to scratch and eval reads the live ones."""
-        B = images.shape[0]
+        B = self._batch_size(images, audios)
         w = self._eval_workspace(B)
         P = self.T if teacher else self.S
         bns = self.bn_t if teacher else self.bn_s
@@ -1050,9 +1115,10 @@ class DinoStepEngine:
             bns = probe["bns"]
         elif train:       # scratch running statistics
             bns = {k: _BN(v.C, self.device) for k, v in bns.items()}
-        xi = w["x_img"]
-        xi.copy_((images.float() / 255.0 if images.dtype == torch.uint8 else images).reshape(B, 1, 28, 28))
-        xa = None
+        xi = xa = None
+        if self.img_layers:
+            xi = w["x_img"]
+            xi.copy_((images.float() / 255.0 if images.dtype == torch.uint8 else images).reshape(B, 1, 28, 28))
         if self.aud_layers:
             xa = w["x_aud"]
             xa.copy_((audios.float() / 255.0 if audios.dtype == torch.uint8 else audios).reshape(B, 1, 112, 112))
@@ -1081,27 +1147,29 @@ class DinoStepEngine:
         through encoders and heads.  Returns the workspace dict; outputs: w['s.proj'] [V*B,P], w['t.proj'] [Vg*B,P]
         (UNcentred), w['aux_image.out'] / w['aux_audio.out'] [B, 10|P]."""
         V, Vg, E = self.V, self.Vg, self.E
-        B = x_img.shape[1]
+        x_in = x_img if self.img_layers else x_aud            # the views of the first encoded modality: [V,B,...]
+        B = x_in.shape[1]
         w = self._workspace(B)
         Ns, Nt, Nv = w["Ns"], w["Nt"], V * B
         S, T = self.S, self.T
         multi = self.multi
-        xi = w["x_img"]
-        xa = w["x_aud"] if multi else None
+        xi = w.get("x_img")
+        xa = w.get("x_aud")
         self._join_center()
         w["zarena"].zero_()                             # all statistics / backward-sum accumulators of this step
-        packed = x_img.dtype == torch.bfloat16          # augment(direct=True): the quad8 workspace images are already filled
+        packed = x_in.dtype == torch.bfloat16           # augment(direct=True): the quad8 workspace images are already filled
         w["packed"] = packed
         if packed:
-            if x_img.data_ptr() != w["img.xs8"].data_ptr() or (multi and x_aud.data_ptr() != w["aud.xs8"].data_ptr()):
+            if ((self.img_layers and x_img.data_ptr() != w["img.xs8"].data_ptr()) or
+                    (self.aud_layers and x_aud.data_ptr() != w["aud.xs8"].data_ptr())):
                 raise ops._lib.B200Error("bf16 inputs must be the workspace quad8 images returned by augment(direct=True)")
             if self.mode != "default":
                 ops.pack_quad8(raw[0].reshape(B, 28, 28), w["img.xs8"][Nv:], self.img_layers[0][6])
                 ops.pack_quad8(raw[1].reshape(B, 112, 112), w["aud.xs8"][Nv:], self.aud_layers[0][6])
         else:
-            if x_img.data_ptr() != xi.data_ptr():
+            if self.img_layers and x_img.data_ptr() != xi.data_ptr():
                 xi[:Nv].copy_(x_img.reshape(Nv, 1, 28, 28))
-            if multi and x_aud.data_ptr() != xa.data_ptr():
+            if self.aud_layers and x_aud.data_ptr() != xa.data_ptr():
                 xa[:Nv].copy_(x_aud.reshape(Nv, 1, 112, 112))
             if self.mode != "default":
                 xi[Nv:].copy_(raw[0].reshape(B, 1, 28, 28))
@@ -1136,14 +1204,14 @@ class DinoStepEngine:
         if side is not None:
             side.wait_stream(main)
             with torch.cuda.stream(side):
-                feat_t = self._encode(w, "t", T, self.bn_t, xi[:Nt], xa[:Nt] if multi else None, Nt, B, Nt, w.get("t.fmask"))
+                feat_t = self._encode(w, "t", T, self.bn_t, _rows(xi, Nt), _rows(xa, Nt), Nt, B, Nt, w.get("t.fmask"))
                 self._head_fwd(w, "t", "head.", T, self.bn_t["head.mlp.1"], feat_t, w["t.proj"], w["t.hh"], w["t.g"], None, 0.0)
         feat_s = self._encode(w, "s", S, self.bn_s, xi, xa, Ns, B, Nv, w.get("s.fmask"))
         self._head_fwd(w, "s", "head.", S, self.bn_s["head.mlp.1"], feat_s, w["s.proj"], w["s.hh"], w["s.g"], w["s.hmask"], self.dropout)
         if side is not None:
             main.wait_stream(side)
         else:
-            feat_t = self._encode(w, "t", T, self.bn_t, xi[:Nt], xa[:Nt] if multi else None, Nt, B, Nt, w.get("t.fmask"))
+            feat_t = self._encode(w, "t", T, self.bn_t, _rows(xi, Nt), _rows(xa, Nt), Nt, B, Nt, w.get("t.fmask"))
             self._head_fwd(w, "t", "head.", T, self.bn_t["head.mlp.1"], feat_t, w["t.proj"], w["t.hh"], w["t.g"], None, 0.0)
         if self.mode != "default":
             cat = w["s.catr"]               # the mode heads read the un-mixed encoder features (models/dino.py:972-980)
@@ -1207,7 +1275,7 @@ class DinoStepEngine:
         Ns, Nv = w["Ns"], V * B
         S, G = self.S, self.G
         multi = self.multi
-        xi, xa = w["x_img"], w.get("x_aud")
+        xi, xa = w.get("x_img"), w.get("x_aud")
         feat_s = w["s.feat"]
         d_proj = w["d.proj"] if d_proj is None else d_proj.reshape(Nv, self.P)
         d_feat = w["d.feat"]
@@ -1215,7 +1283,7 @@ class DinoStepEngine:
         if self.cosine_loss_alpha > 0:
             ops.cosine_consistency_fwd_bwd(feat_s.view(V, B, O), w["d.emb"].view(V, B, O), w["loss"][2:3], grad_scale=self.cosine_loss_alpha,
                                            work=w["loss_work"])
-            d_feat.add_(w["d.emb"])
+            ops.add2d(d_feat, w["d.emb"])
         if multi:
             d_cat, d_catr, d_h1 = w["d.cat"], w["d.catr"], w["d.h1"]
             self._lin_wgrad(d_feat, w["s.h1"], G["enc.fusion.3.weight"], G["enc.fusion.3.bias"])
@@ -1254,13 +1322,16 @@ class DinoStepEngine:
             if side is not None:
                 main.wait_stream(side)
         else:
-            self._lin_wgrad(d_feat, w["s.e14"], G["enc.projection.0.weight"], G["enc.projection.0.bias"])
-            ops.linear_bwd_data(d_feat, S["enc.projection.0.weight"], w["d.e14"], tc=self.lin_tc)
-            self._lin_wgrad(w["d.e14"], w["s.pool"], G["enc.encoder.14.weight"], G["enc.encoder.14.bias"])
-            ops.linear_bwd_data(w["d.e14"], S["enc.encoder.14.weight"], w["d.pool"], tc=self.lin_tc)
-            d_p = w["img.dp_a"][:Ns * 128 * 9].view(Ns, 128, 3, 3)
+            mod, _, chain = self.uni
+            layers = self._layers(mod)
+            for lin, src, dst, _ in reversed(chain):
+                d_out = d_feat if dst == "feat" else w[f"d.{dst}"]
+                self._lin_wgrad(d_out, w[f"s.{src}"], G[lin + ".weight"], G[lin + ".bias"])
+                ops.linear_bwd_data(d_out, S[lin + ".weight"], w[f"d.{src}"], tc=self.lin_tc)
+            p_last = w[f"s.{mod}.p{len(layers) - 1}"]
+            d_p = w[f"{mod}.dp_a"][:p_last.numel()].view_as(p_last)
             ops.avgpool_bwd(w["d.pool"], d_p)
-            self._conv_stack_bwd(w, "img", self.img_layers, xi, d_p, Ns, B)
+            self._conv_stack_bwd(w, mod, layers, xi if mod == "img" else xa, d_p, Ns, B)
         if self._lin_wg_pending:
             torch.cuda.current_stream().wait_stream(self._lin_wg_stream)
             self._lin_wg_pending = False
@@ -1406,7 +1477,9 @@ class DinoStepEngine:
         lock-step.  The learning rate is a device scalar (schedulers may change engine.lr between replays); temperatures, momenta and
         weight decay are baked in (re-capture after changing them).  Use graph_step() afterwards."""
         dev = self.device
-        g = {"B": B, "img": torch.zeros(B, 28, 28, dtype=image_dtype, device=dev)}
+        g = {"B": B}
+        if self.img_layers:
+            g["img"] = torch.zeros(B, 28, 28, dtype=image_dtype, device=dev)
         if self.aud_layers:
             g["aud"] = torch.zeros(B, 112, 112, dtype=audio_dtype, device=dev)
         if self.mode == "semi_supervised":
@@ -1421,7 +1494,7 @@ class DinoStepEngine:
         self._graph_lr = float(self.lr)
 
         def body():
-            return self.train_step(g["img"], g.get("aud"), g.get("lab"))
+            return self.train_step(g.get("img"), g.get("aud"), g.get("lab"))
 
         def restore():
             for t, c in zip(state, snap):
@@ -1451,9 +1524,10 @@ class DinoStepEngine:
     def graph_step(self, images, audios=None, labels=None):
         """One training step by replaying the captured graph on a raw device batch; returns the device loss tensor [4]."""
         g = self._graph
-        if g is None or images.shape[0] != g["B"]:
+        if g is None or self._batch_size(images, audios) != g["B"]:
             raise ops._lib.B200Error("graph_step: call capture_train_step(B) for this batch size first")
-        g["img"].copy_(images.reshape(g["img"].shape))
+        if "img" in g:
+            g["img"].copy_(images.reshape(g["img"].shape))
         if "aud" in g:
             g["aud"].copy_(audios.reshape(g["aud"].shape))
         if "lab" in g:
@@ -1488,43 +1562,45 @@ class DinoStepEngine:
         step's loss is read back, so the input pipeline overlaps the step (what the reference's DataLoader workers do).
         lagged_loss=True: every step's loss is still copied to (pinned) host memory, but the call returns the PREVIOUS step's
         value (None on the first call; flush_loss() returns the last one) so that the host never waits for the step it has
-        just enqueued -- the usual way a training loop logs its loss."""
-        B = images_host.shape[0]
-        buf = self._ws.setdefault(("host", B, images_host.dtype, None if audios_host is None else audios_host.dtype), {})
+        just enqueued -- the usual way a training loop logs its loss.  An audio-only kind ignores the image batches (they may be None)."""
+        def ptr(t):
+            return None if t is None else t.data_ptr()
+
+        if not self.img_layers:
+            images_host = None
+            if next_batch is not None:
+                next_batch = (None,) + tuple(next_batch[1:])
+        B = self._batch_size(images_host, audios_host)
+        buf = self._ws.setdefault(("host", B, None if images_host is None else images_host.dtype,
+                                   None if audios_host is None else audios_host.dtype), {})
         if not buf:
             for tag in ("", "_b"):
-                buf["img" + tag] = torch.empty(images_host.shape, dtype=images_host.dtype, device=self.device)
-                if audios_host is not None:
-                    buf["aud" + tag] = torch.empty(audios_host.shape, dtype=audios_host.dtype, device=self.device)
-                if labels_host is not None:
-                    buf["lab" + tag] = torch.empty(labels_host.shape, dtype=labels_host.dtype, device=self.device)
+                for k, t in (("img", images_host), ("aud", audios_host), ("lab", labels_host)):
+                    if t is not None:
+                        buf[k + tag] = torch.empty(t.shape, dtype=t.dtype, device=self.device)
             buf["staged"] = None
-        if buf["staged"] is not None and buf["staged"] == (images_host.data_ptr(), None if audios_host is None else audios_host.data_ptr()):
+        if buf["staged"] is not None and buf["staged"] == (ptr(images_host), ptr(audios_host)):
             for k in ("img", "aud", "lab"):                       # this batch was staged by the previous call: swap the slots
                 if k in buf:
                     buf[k], buf[k + "_b"] = buf[k + "_b"], buf[k]
         else:
             self._prefetch = None
-            buf["img"].copy_(images_host, non_blocking=True)
-            if audios_host is not None:
-                buf["aud"].copy_(audios_host, non_blocking=True)
-            if labels_host is not None:
-                buf["lab"].copy_(labels_host, non_blocking=True)
+            for k, t in (("img", images_host), ("aud", audios_host), ("lab", labels_host)):
+                if t is not None:
+                    buf[k].copy_(t, non_blocking=True)
         buf["staged"] = None
-        loss = self.train_step(buf["img"], buf.get("aud"), buf.get("lab"))
+        loss = self.train_step(buf.get("img"), buf.get("aud"), buf.get("lab"))
         if next_batch is not None:
             nimg, naud = next_batch[0], (next_batch[1] if len(next_batch) > 1 else None)
             nlab = next_batch[2] if len(next_batch) > 2 else None
             with torch.cuda.stream(self._aug_stream):
                 if self._step_done_prev is not None:
                     self._aug_stream.wait_event(self._step_done_prev)      # the spare raw buffers were last read one step back
-                buf["img_b"].copy_(nimg, non_blocking=True)
-                if naud is not None:
-                    buf["aud_b"].copy_(naud, non_blocking=True)
-                if nlab is not None:
-                    buf["lab_b"].copy_(nlab, non_blocking=True)
-            if self.prefetch_augment(buf["img_b"], buf.get("aud_b")):
-                buf["staged"] = (nimg.data_ptr(), None if naud is None else naud.data_ptr())
+                for k, t in (("img", nimg), ("aud", naud), ("lab", nlab)):
+                    if t is not None:
+                        buf[k + "_b"].copy_(t, non_blocking=True)
+            if self.prefetch_augment(buf.get("img_b"), buf.get("aud_b")):
+                buf["staged"] = (ptr(nimg), ptr(naud))
         if not lagged_loss:
             return float(loss[3].item())
         prev = self.flush_loss()
