@@ -6,7 +6,7 @@ import subprocess
 MULTIMODAL = ["multi_simple", "multi_simple_gated", "multi_lstm", "multi_vit", "multi_dual_vit", "multi_mobile_vit", "multi_resnet",
               "multi_cross_attention", "multi_central"]
 UNIMODAL = ["image_simple", "spectrogram_simple", "spectrogram_central", "spectrogram_lstm", "spectrogram_resnet", "spectrogram_vit",
-            "spectrogram_mobile_vit"]
+            "spectrogram_mobile_vit", "image_central"]
 
 
 def main(argv=None):

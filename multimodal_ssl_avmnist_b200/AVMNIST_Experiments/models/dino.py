@@ -7,10 +7,11 @@ Adam -- runs in hand-written sm_100a kernels behind libavmnist_b200.so (multimod
 There is no PyTorch fallback: on a CPU tensor, or without the library, the step raises.
 
 Compiled encoders: CentralMultiModalEncoder ("multi_central"), the conv encoders SimpleMultiModalEncoder ("multi_simple"),
-GatedMultiModalEncoder ("multi_simple_gated") and CrossAttentionMultiModalEncoder ("multi_cross_attention") (SURVEY 8f-4), and the
-unimodal ImageEncoder ("image_simple") and SpectrogramEncoder ("spectrogram_simple").  The other encoder families of the reference
-(LSTM, ViT, MobileViT, ResNet, the other spectrogram encoders) are outside the hot-path scope; their names exist so that driver
-scripts import, and constructing one raises NotImplementedError.
+GatedMultiModalEncoder ("multi_simple_gated") and CrossAttentionMultiModalEncoder ("multi_cross_attention") (SURVEY 8f-4), the
+unimodal ImageEncoder ("image_simple") and SpectrogramEncoder ("spectrogram_simple"), and the unimodal LeNet-style CentralNet encoders
+ImageEncoderCentral ("image_central") and SpectrogramEncoderCentral ("spectrogram_central").  The other encoder families of the
+reference (LSTM, ViT, MobileViT, ResNet, the other spectrogram encoders) are outside the hot-path scope; their names exist so that
+driver scripts import, and constructing one raises NotImplementedError.
 """
 import os
 import sys
@@ -201,15 +202,52 @@ class SpectrogramEncoder(BaseUniModalEncoder):
         return MF.sequential_cnn_forward(self.encoder, spectrograms)
 
 
+class ImageEncoderCentral(BaseUniModalEncoder):
+    """The image branch of CentralMultiModalEncoder alone: encoder = Sequential(CentralUnimodalImage (2 x conv5; fc1 / fc2 unused),
+    Linear(64*5*5, output_dim)) on the flattened 64x5x5 activation -- the image-only DINO encoder of the LeNet family
+    (`--unimodal_model image_central`).  The reference has no LeNet unimodal image class: this layout copies
+    CentralMultiModalEncoder's image branch under `encoder.`; it is not pinned against a reference checkpoint."""
+    B200_KIND = "image_central"
+
+    def __init__(self, output_dim=256):
+        super().__init__(output_dim, modality="image")
+        self.encoder = _HeadedCNN(CentralUnimodalImage(), nn.Linear(64 * 5 * 5, output_dim))
+
+    def forward(self, images=None, spectrograms=None):
+        if images is None:
+            raise ValueError("ImageEncoderCentral requires image input")
+        return self.encoder(images)
+
+
+class SpectrogramEncoderCentral(BaseUniModalEncoder):
+    """The audio branch of CentralMultiModalEncoder alone: encoder = Sequential(CentralUnimodalAudio (4 x conv5; fc1 / fc2 unused),
+    Linear(64*7*7, output_dim)) on the flattened 64x7x7 activation (`--unimodal_model spectrogram_central`).  The body of the
+    reference's SpectrogramEncoderCentral is not available here: this layout copies CentralMultiModalEncoder's audio branch under
+    `encoder.`, so reference checkpoints of this class are not known to load strictly."""
+    B200_KIND = "spectrogram_central"
+
+    def __init__(self, output_dim=256):
+        super().__init__(output_dim, modality="audio")
+        self.encoder = _HeadedCNN(CentralUnimodalAudio(), nn.Linear(64 * 7 * 7, output_dim))
+
+    def forward(self, images=None, spectrograms=None):
+        if spectrograms is None:
+            raise ValueError("SpectrogramEncoderCentral requires spectrogram input")
+        return self.encoder(spectrograms)
+
+
+_COMPILED = ("Central / Simple / Gated / CrossAttention MultiModalEncoder, ImageEncoder, SpectrogramEncoder, ImageEncoderCentral, "
+             "SpectrogramEncoderCentral")
+
+
 def _out_of_scope(name):
     def __init__(self, *a, **k):
-        raise NotImplementedError(f"{name} is outside the B200 hot-path scope (see DESIGN.md section 7); "
-                                  "compiled encoders: Central / Simple / Gated / CrossAttention MultiModalEncoder, ImageEncoder, SpectrogramEncoder")
+        raise NotImplementedError(f"{name} is outside the B200 hot-path scope (see DESIGN.md section 7); compiled encoders: {_COMPILED}")
     return type(name, (nn.Module,), {"__init__": __init__, "B200_KIND": None})
 
 
 for _n in ("LSTMImageEncoder", "LSTMMultiModalEncoder", "ViTMultiModalEncoder", "DualViTMultiModalEncoder", "MobileViTMultiModalEncoder",
-           "ResNetMultiModalEncoder", "SpectrogramEncoderCentral", "SpectrogramEncoderLSTM", "SpectrogramEncoderResNet", "SpectrogramEncoderViT",
+           "ResNetMultiModalEncoder", "SpectrogramEncoderLSTM", "SpectrogramEncoderResNet", "SpectrogramEncoderViT",
            "SpectrogramEncoderMobileViT", "UniModalDINOV2"):
     globals()[_n] = _out_of_scope(_n)
 
@@ -251,8 +289,7 @@ class _DinoBase(nn.Module):
         self.register_buffer("center", torch.zeros(1, projection_dim))
         kind = getattr(encoder_class, "B200_KIND", None)
         if kind is None:
-            raise NotImplementedError(f"{encoder_class.__name__} has no compiled B200 training step "
-                                      "(compiled: Central / Simple / Gated / CrossAttention MultiModalEncoder, ImageEncoder, SpectrogramEncoder)")
+            raise NotImplementedError(f"{encoder_class.__name__} has no compiled B200 training step (compiled: {_COMPILED})")
         self._b200 = B.EngineBinding(self, kind, self.MODE)
         self.student_temperature, self.teacher_temperature = 0.1, 0.04
         self.n_global_views, self.n_local_views = 2, 4

@@ -27,7 +27,7 @@ from _compat import CSVLogger, ModelCheckpoint, pl  # noqa: E402
 from configs.update_config import update_hardware_config  # noqa: E402
 from hyperparameter_tuning.objective_augment import process_augment_config  # noqa: E402
 from models.dino import (CentralMultiModalEncoder, CrossAttentionMultiModalEncoder, DualViTMultiModalEncoder, GatedMultiModalEncoder,  # noqa: E402
-                         ImageEncoder, LSTMMultiModalEncoder, MobileViTMultiModalEncoder, MultiModalDINOLightning,
+                         ImageEncoder, ImageEncoderCentral, LSTMMultiModalEncoder, MobileViTMultiModalEncoder, MultiModalDINOLightning,
                          MultiModalDINOSemiSupervisedLightning, MultiModalDINOWithINFONCELightning, MultiModalDINOWithMSELightning,
                          ResNetMultiModalEncoder, SimpleMultiModalEncoder, SpectrogramEncoder, SpectrogramEncoderCentral,
                          SpectrogramEncoderLSTM, SpectrogramEncoderMobileViT, SpectrogramEncoderResNet, SpectrogramEncoderViT,
@@ -41,7 +41,8 @@ MODEL_MAP = {"multi_simple": SimpleMultiModalEncoder, "multi_simple_gated": Gate
              "multi_central": CentralMultiModalEncoder}
 UNIMODAL_MODEL_MAP = {"image_simple": ImageEncoder, "spectrogram_simple": SpectrogramEncoder, "spectrogram_central": SpectrogramEncoderCentral,
                       "spectrogram_lstm": SpectrogramEncoderLSTM, "spectrogram_resnet": SpectrogramEncoderResNet,
-                      "spectrogram_vit": SpectrogramEncoderViT, "spectrogram_mobile_vit": SpectrogramEncoderMobileViT}
+                      "spectrogram_vit": SpectrogramEncoderViT, "spectrogram_mobile_vit": SpectrogramEncoderMobileViT,
+                      "image_central": ImageEncoderCentral}
 MULTIMODAL_WRAPPERS = {"default": MultiModalDINOLightning, "semi_supervised": MultiModalDINOSemiSupervisedLightning,
                        "mse": MultiModalDINOWithMSELightning, "infonce": MultiModalDINOWithINFONCELightning}
 

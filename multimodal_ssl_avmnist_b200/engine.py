@@ -14,9 +14,10 @@ streams; for data parallel runs the two exchanges (gradient arena, centre column
 
 Encoders (`kind`): 'multi_central' (CentralMultiModalEncoder, the headline), 'multi_simple' / 'multi_simple_gated' /
 'multi_cross_attention' (the 3x3 conv encoders of models/dino.py:214-263, 385-452: stack tops are avgpool -> linear and a mix stage --
-sigmoid gates or batch-wide cross attention -- sits before the fusion MLP), and the unimodal 'image_simple' (ImageEncoder) and
-'spectrogram_simple' (SpectrogramEncoder: the audio stack of 'multi_simple' alone).  The stand-alone contrastive
-steps of other_ssl/ reuse these building blocks from contrastive.ContrastiveStepEngine.
+sigmoid gates or batch-wide cross attention -- sits before the fusion MLP), the unimodal 'image_simple' (ImageEncoder) and
+'spectrogram_simple' (SpectrogramEncoder: the audio stack of 'multi_simple' alone), and the unimodal CentralNet kinds 'image_central'
+(ImageEncoderCentral) and 'spectrogram_central' (SpectrogramEncoderCentral): one branch of 'multi_central' each, flatten -> Linear to
+the embedding.  The stand-alone contrastive steps of other_ssl/ reuse these building blocks from contrastive.ContrastiveStepEngine.
 
 Arena layout (student):  [ encoder params that receive gradients | projection head | unused fc1/fc2 | mode heads ]
         (teacher):       [ encoder params that receive gradients | projection head | unused fc1/fc2 ]
@@ -99,6 +100,25 @@ def spectrogram_simple_params(O):
     return used, []
 
 
+def _central_branch_params(branch, O):
+    """One branch of CentralMultiModalEncoder alone under `encoder.` (ImageEncoderCentral / SpectrogramEncoderCentral):
+    encoder.0 = the CentralUnimodal CNN (conv{k}, bn{k}; fc1 / fc2 unused), encoder.1 = Linear(flat, O) -> the embedding."""
+    pre = f"{branch}_encoder."
+
+    def take(specs):
+        return [("encoder." + n[len(pre):], s) for n, s in specs if n.startswith(pre)]
+    used, unused = central_encoder_params(O, O)
+    return take(used), take(unused)
+
+
+def image_central_params(O):
+    return _central_branch_params("image", O)
+
+
+def spectrogram_central_params(O):
+    return _central_branch_params("audio", O)
+
+
 def simple_multi_params(E, O, mix=None):
     """Parameter specs of SimpleMultiModalEncoder (models/dino.py:214-234: image_encoder() / audio_encoder() `nn.Sequential`s,
     :18-73, + the concatenation fusion) and its two subclasses: GatedMultiModalEncoder (:237-263, two scalar gates) and
@@ -137,12 +157,24 @@ MULTI_SIMPLE_AUDIO_LAYERS = [("audio_encoder.0", "audio_encoder.1", 1, 32, 112, 
                              ("audio_encoder.8", "audio_encoder.9", 64, 128, 28, 3, 1), ("audio_encoder.12", "audio_encoder.13", 128, 256, 14, 3, 1)]
 SPECTROGRAM_LAYERS = [("encoder.0", "encoder.1", 1, 32, 112, 3, 1), ("encoder.4", "encoder.5", 32, 64, 56, 3, 1),
                       ("encoder.8", "encoder.9", 64, 128, 28, 3, 1), ("encoder.12", "encoder.13", 128, 256, 14, 3, 1)]
+
+
+def _reprefix(layers, old, new):
+    return [(conv.replace(old, new, 1), bn.replace(old, new, 1), *geom) for conv, bn, *geom in layers]
+
+
+# the unimodal CentralNet kinds: the branches of multi_central under `encoder.`
+CENTRAL_IMAGE_UNI_LAYERS = _reprefix(CENTRAL_IMAGE_LAYERS, "image_encoder.", "encoder.")
+CENTRAL_AUDIO_UNI_LAYERS = _reprefix(CENTRAL_AUDIO_LAYERS, "audio_encoder.", "encoder.")
 # kind -> feature mixing between the encoders and the fusion MLP
 MULTI_KINDS = {"multi_central": None, "multi_simple": None, "multi_simple_gated": "gated", "multi_cross_attention": "cross"}
-# unimodal kind -> (modality stack, width of the global average pool, [(linear, input buffer, output buffer, output width)] after the
-# pool; the last output is the embedding `feat` that the projection head and the cosine-consistency term read)
-UNI_KINDS = {"image_simple": ("img", 128, [("enc.encoder.14", "pool", "e14", 512), ("enc.projection.0", "e14", "feat", None)]),
-             "spectrogram_simple": ("aud", 256, [("enc.encoder.18", "pool", "feat", None)])}
+# unimodal kind -> (modality stack, stack top, [(linear, input buffer, output buffer, output width)] after the top; the last output is
+# the embedding `feat` that the projection head and the cosine-consistency term read).  The top is ("pool", W): global average pool to
+# W features, or ("flat", W): the last pooled activation flattened to W = C*h*w features; either way the buffer "top" [N, W] holds them
+UNI_KINDS = {"image_simple": ("img", ("pool", 128), [("enc.encoder.14", "top", "e14", 512), ("enc.projection.0", "e14", "feat", None)]),
+             "spectrogram_simple": ("aud", ("pool", 256), [("enc.encoder.18", "top", "feat", None)]),
+             "image_central": ("img", ("flat", 64 * 5 * 5), [("enc.encoder.1", "top", "feat", None)]),
+             "spectrogram_central": ("aud", ("flat", 64 * 7 * 7), [("enc.encoder.1", "top", "feat", None)])}
 
 
 class Arena:
@@ -201,7 +233,8 @@ def _main_chain(fn):
 class DinoStepEngine:
     """See module docstring.  kind: 'multi_central' (CentralMultiModalEncoder), 'multi_simple' (SimpleMultiModalEncoder),
     'multi_simple_gated' (GatedMultiModalEncoder), 'multi_cross_attention' (CrossAttentionMultiModalEncoder), 'image_simple'
-    (ImageEncoder) or 'spectrogram_simple' (SpectrogramEncoder); mode: 'default' | 'semi_supervised' | 'infonce' | 'mse' (multimodal
+    (ImageEncoder), 'spectrogram_simple' (SpectrogramEncoder), 'image_central' (ImageEncoderCentral) or 'spectrogram_central'
+    (SpectrogramEncoderCentral); mode: 'default' | 'semi_supervised' | 'infonce' | 'mse' (multimodal
     kinds only).  The unimodal kinds have one conv stack; the methods that take (images, audios) ignore the absent modality's
     argument (it may be None) and allocate nothing for it."""
 
@@ -254,11 +287,19 @@ class DinoStepEngine:
             used, unused = image_simple_params(self.O)
             self.img_layers, self.aud_layers = SIMPLE_IMAGE_LAYERS, []
             self.top = {}
-        else:
+        elif kind == "spectrogram_simple":
             used, unused = spectrogram_simple_params(self.O)
             self.img_layers, self.aud_layers = [], SPECTROGRAM_LAYERS
             self.top = {}
-        # unimodal kinds: the modality of the one conv stack and the layers between its global average pool and the embedding
+        elif kind == "image_central":
+            used, unused = image_central_params(self.O)
+            self.img_layers, self.aud_layers = CENTRAL_IMAGE_UNI_LAYERS, []
+            self.top = {}
+        else:
+            used, unused = spectrogram_central_params(self.O)
+            self.img_layers, self.aud_layers = [], CENTRAL_AUDIO_UNI_LAYERS
+            self.top = {}
+        # unimodal kinds: the modality of the one conv stack, its top and the layers between the top and the embedding
         self.uni = UNI_KINDS.get(kind)
         head = [("head." + n, s) for n, s in head_params(self.O, self.P)]
         enc_used = [("enc." + n, s) for n, s in used]
@@ -311,8 +352,9 @@ class DinoStepEngine:
         # layers keep the z -> bn_relu_pool8_fwd path.  self.pool[role][mod][li]; role "t" also serves evaluation.
         # False: the round-1 path everywhere (A/B measurements).  The simple encoder family keeps it off: its layers are 32 - 256 channels
         # wide, and the per-tile barrier + the wider pooled rows cost the epilogue far more than the z read saves (first audio layer,
-        # 32 channels at 112x112: 2.86 ms fused against 0.96 + 1.15 ms conv + pool pass; whole step 26.1 vs 25.1 ms, profiles/r2zf_*)
-        self.fused_pool = bool(fused_pool) and kind in ("multi_central", "image_simple")
+        # 32 channels at 112x112: 2.86 ms fused against 0.96 + 1.15 ms conv + pool pass; whole step 26.1 vs 25.1 ms, profiles/r2zf_*).
+        # The unimodal CentralNet kinds run multi_central's layers and take its policy
+        self.fused_pool = bool(fused_pool) and kind in ("multi_central", "image_simple", "image_central", "spectrogram_central")
         self.pool = {}
         for role in ("s", "t"):
             self.pool[role] = {mod: [self.fused_pool and bool(self.tc[mod][li]) and ops.conv_tc_pool_supported(ci, co, hw, hw, k, pad)
@@ -595,9 +637,16 @@ class DinoStepEngine:
         return w
 
     def _uni_workspace(self, w, role, N, e, with_feat=True):
-        """Unimodal kinds: the pooled features [N, pool width] and the outputs of the linears after the pool (`feat` [N, O] last)."""
-        _, width, chain = self.uni
-        w[f"{role}.pool"] = e(N, width)
+        """Unimodal kinds: the stack's top features "top" [N, W] and the outputs of the linears after it (`feat` [N, O] last).  An
+        average-pool top has its own buffer; a flatten top is a view of the last pooled activation (role "d": of the gradient buffer
+        dp_a that the stack's backward starts from, so that the first linear's data gradient lands there directly)."""
+        mod, (top, width), chain = self.uni
+        if top == "pool":
+            w[f"{role}.top"] = e(N, width)
+        elif role == "d":
+            w["d.top"] = w[f"{mod}.dp_a"][:N * width].view(N, width)
+        else:
+            w[f"{role}.top"] = w[f"{role}.{mod}.p{len(self._layers(mod)) - 1}"].view(N, width)
         for lin, src, dst, cols in chain:
             if dst != "feat" or with_feat:
                 w[f"{role}.{dst}"] = e(N, self.O if cols is None else cols)
@@ -931,10 +980,12 @@ class DinoStepEngine:
                 ops.linear_fwd(cat[:n_fusion], P["enc.fusion.0.weight"], P["enc.fusion.0.bias"], h1, act=2, mask=fmask, drop_p=self.fusion_dropout, tc=self.lin_tc)
             ops.linear_fwd(h1, P["enc.fusion.3.weight"], P["enc.fusion.3.bias"], feat, tc=self.lin_tc)
             return feat
-        # unimodal: conv stack -> global average pool -> the linears of self.uni (image: encoder.14, projection.0; audio: encoder.18)
-        mod, _, chain = self.uni
+        # unimodal: conv stack -> top (global average pool, or flatten: w[role.top] is already a view of p_last) -> the linears of
+        # self.uni (image_simple: encoder.14, projection.0; spectrogram_simple: encoder.18; the CentralNet kinds: encoder.1)
+        mod, (top, _), chain = self.uni
         p_last = self._conv_stack(w, role, mod, self._layers(mod), x_img if mod == "img" else x_aud, N, B, P, bns, train=train)
-        ops.avgpool_fwd(p_last, w[f"{role}.pool"])
+        if top == "pool":
+            ops.avgpool_fwd(p_last, w[f"{role}.top"])
         for lin, src, dst, _ in chain:
             ops.linear_fwd(w[f"{role}.{src}"], P[lin + ".weight"], P[lin + ".bias"], w[f"{role}.{dst}"], tc=self.lin_tc)
         return w[f"{role}.feat"]
@@ -1322,15 +1373,18 @@ class DinoStepEngine:
             if side is not None:
                 main.wait_stream(side)
         else:
-            mod, _, chain = self.uni
+            mod, (top, _), chain = self.uni
             layers = self._layers(mod)
             for lin, src, dst, _ in reversed(chain):
                 d_out = d_feat if dst == "feat" else w[f"d.{dst}"]
                 self._lin_wgrad(d_out, w[f"s.{src}"], G[lin + ".weight"], G[lin + ".bias"])
                 ops.linear_bwd_data(d_out, S[lin + ".weight"], w[f"d.{src}"], tc=self.lin_tc)
-            p_last = w[f"s.{mod}.p{len(layers) - 1}"]
-            d_p = w[f"{mod}.dp_a"][:p_last.numel()].view_as(p_last)
-            ops.avgpool_bwd(w["d.pool"], d_p)
+            if top == "pool":
+                p_last = w[f"s.{mod}.p{len(layers) - 1}"]
+                d_p = w[f"{mod}.dp_a"][:p_last.numel()].view_as(p_last)
+                ops.avgpool_bwd(w["d.top"], d_p)
+            else:                       # flatten: the first linear's data gradient already is the stack's top gradient (in dp_a)
+                d_p = w["d.top"]
             self._conv_stack_bwd(w, mod, layers, xi if mod == "img" else xa, d_p, Ns, B)
         if self._lin_wg_pending:
             torch.cuda.current_stream().wait_stream(self._lin_wg_stream)
