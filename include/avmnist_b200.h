@@ -351,6 +351,14 @@ int b200_adam_flat_dev(float* param, const float* grad, float* exp_avg, float* e
                        float beta1, float beta2, float eps, float weight_decay, const float* bc_dev, float grad_scale,
                        void* stream);
 int b200_counters_advance(int64_t* counters, int n, void* stream);
+/* torch.optim.AdamW over one flat arena (decoupled weight decay): p <- p * (1 - lr*weight_decay), then the Adam update of
+ * b200_adam_flat with no L2 term.  With weight_decay = 0 the result is bit-identical to b200_adam_flat.  The _dev variant reads
+ * the bias corrections (and, with lr < 0, the learning rate) from bc_dev like b200_adam_flat_dev, for CUDA-graph replay. */
+int b200_adamw_flat(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, int64_t n, float lr,
+                    float beta1, float beta2, float eps, float weight_decay, float bias_correction1,
+                    float bias_correction2_sqrt, void* stream);
+int b200_adamw_flat_dev(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, int64_t n, float lr,
+                        float beta1, float beta2, float eps, float weight_decay, const float* bc_dev, void* stream);
 /* y <- y * alpha (used to apply an upstream autograd scale / the 1/world_size of the gradient all-reduce) */
 int b200_scale_flat(float* y, int64_t n, float alpha, void* stream);
 
@@ -367,6 +375,24 @@ int b200_scale_flat(float* y, int64_t n, float alpha, void* stream);
 int b200_knn_neg_half_sqnorm(const float* x, int64_t ldx, int N, int D, float* out, void* stream);
 int b200_knn_topk_vote(const float* scores, int64_t lds, const int64_t* labels, int M, int N, int k, int n_classes,
                        int64_t* pred, int32_t* neighbours, void* stream);
+
+/* ------------------------------------------------------------------------------------------------------------
+ * Downstream MLP probe on frozen features (train_downstream, training_structures/dino_train.py): the DownstreamClassifier head
+ * Linear(O, 128) -> ReLU -> Linear(128, C) with nn.CrossEntropyLoss (mean over the batch), fp32 throughout.
+ *   x [B, O] features (O in 64..1024, a multiple of 4), w1 [128, O], b1 [128], w2 [C, 128], b2 [C] (C in 1..16), labels int64 [B]
+ *   in [0, C) (a label outside it makes the batch's loss NaN and is left out of the counts).
+ *   train = 1: grad = float[128*O + 128 + 128*C + C] laid out as [dW1 | db1 | dW2 | db2] (the parameter arena's order) is
+ *     WRITTEN (not accumulated); every weight / bias gradient is a sum over the batch in a fixed order (no float atomics), so two
+ *     runs are bit-identical.
+ *   train = 0: forward only; preds (int64 [B], may be NULL) receives the argmax (first maximum, as torch.argmax), and confusion
+ *     (int64 [C, C], may be NULL) gets += 1 at [label, pred] per row.
+ *   Both: *loss_sum += the batch's loss SUM (fp64, fixed order), *correct += the number of rows whose argmax equals the label.
+ *   work: float[b200_probe_work_floats(B, C)], 16-byte aligned, contents irrelevant on entry.  Two launches.
+ * ---------------------------------------------------------------------------------------------------------- */
+int64_t b200_probe_work_floats(int B, int C);
+int b200_probe_mlp_fwd_bwd(const float* x, const float* w1, const float* b1, const float* w2, const float* b2, const int64_t* labels,
+                           int B, int O, int C, int train, float* grad, float* work, double* loss_sum, int64_t* correct,
+                           int64_t* preds, int64_t* confusion, void* stream);
 
 /* ------------------------------------------------------------------------------------------------------------
  * Feature mixing of the "simple" multimodal encoder family (SURVEY 8f-4), between the per-modality encoders and the fusion MLP:

@@ -4,13 +4,15 @@
     python run_dino.py --unimodal_model image_simple --config config_multimodal_dino.yaml
 
 It builds the same Lightning module with the same keyword arguments, the same data module and Trainer arguments and runs the
-3-seed training loop on the B200 step.  Out of scope (DESIGN.md section 1): Optuna searches, GFLOPs tables, downstream kNN / MLP
-evaluation, plots.  `--synthetic N` writes an AVMNIST-shaped synthetic data set first (smoke runs without the real files);
-`--max_steps` bounds each seed's run.  For N GPUs launch one process per GPU:
+3-seed training loop on the B200 step.  Out of scope (DESIGN.md section 1): Optuna searches, GFLOPs tables, plots.
+`--evaluate` runs the reference's post-training evaluation after each seed (compute_accuracies: kNN + the 10-epoch MLP probe on
+the device, DESIGN.md section 4.11) and adds knn_acc / mlp_acc to the summary.  `--synthetic N` writes an AVMNIST-shaped
+synthetic data set first (smoke runs without the real files); `--max_steps` bounds each seed's run.  For N GPUs launch one process per GPU:
     torchrun --nproc-per-node N run_dino.py --model multi_central --config ...
 """
 import argparse
 import copy
+import json
 import os
 import shutil
 import sys
@@ -79,8 +81,22 @@ class ModelStatsCallback(pl.Callback):
         trainer.callback_metrics["total_training_time"] = time.time() - self.t0
 
 
+def evaluate_seed(model, data, model_dir_data, seed):
+    """compute_accuracies (kNN + MLP probe + metrics) of the just-trained student on the labelled train split and the test split
+    of the run's data; writes downstream_metrics_seed{seed}.json and returns {"knn_acc", "mlp_acc"}."""
+    from training_structures.dino_train import compute_accuracies
+    if getattr(data, "test_dataset", None) is None:
+        data.setup("test")
+    res = compute_accuracies(model.model, data.probe_dataloaders()[0], data.test_dataloader())
+    metrics = {k: (v.tolist() if hasattr(v, "tolist") else v) for k, v in res["metrics"].items()}
+    os.makedirs(model_dir_data, exist_ok=True)
+    with open(os.path.join(model_dir_data, f"downstream_metrics_seed{seed}.json"), "w") as f:
+        json.dump({"seed": seed, "knn_acc": res["knn_acc"], "mlp_acc": res["mlp_acc"], "metrics": metrics}, f, indent=1)
+    return {"knn_acc": res["knn_acc"], "mlp_acc": res["mlp_acc"]}
+
+
 def experiment(config, model, ModelClass, model_name, model_dir_scratch, model_dir_data, extended_data_module=False, study=None,
-               max_steps=-1, seeds=(1, 2, 3)):
+               max_steps=-1, seeds=(1, 2, 3), evaluate=False):
     initial = copy.deepcopy(model.state_dict())
     hp = config["hyperparameters"]
     augments = MultiModalAugmentation(augment_values=process_augment_config(None, config, is_hyperparameter_search=False))
@@ -107,11 +123,18 @@ def experiment(config, model, ModelClass, model_name, model_dir_scratch, model_d
         m = trainer.callback_metrics
         results.append({"seed": seed, "train_loss": float(m.get("train_loss", float("nan"))), "training_time_s": time.time() - t0,
                         "avg_batch_time": float(m.get("avg_batch_time", float("nan")))})
+        if evaluate:
+            results[-1].update(evaluate_seed(model, data, model_dir_data, seed))
     os.makedirs(model_dir_data, exist_ok=True)
     with open(os.path.join(model_dir_data, "performance_summary.txt"), "w") as f:
         f.write(f"model_name: {config['model']['name']}\n")
         for r in results:
             f.write(", ".join(f"{k}: {v}" for k, v in r.items()) + "\n")
+        if evaluate:
+            import numpy as np
+            for key in ("knn_acc", "mlp_acc"):
+                vals = np.array([r[key] for r in results], dtype=np.float64)
+                f.write(f"{key}: {vals.mean():.4f} ± {vals.std():.4f} (mean ± std over seeds)\n")
         f.write("\n# Augmentation Summary\n" + str(data.augmentations) + "\n")
     return results
 
@@ -129,6 +152,7 @@ def main(argv=None):
     ap.add_argument("--synthetic", type=int, default=0, help="write N synthetic AVMNIST-shaped training samples into data_dir first")
     ap.add_argument("--max_steps", type=int, default=-1)
     ap.add_argument("--seeds", type=int, nargs="*", default=[1, 2, 3])
+    ap.add_argument("--evaluate", action="store_true", help="after each seed: kNN + MLP-probe accuracy (compute_accuracies)")
     args = ap.parse_args(argv)
     if args.unimodal_model and args.training_mode != "default":
         raise ValueError(f"--training_mode '{args.training_mode}' is only compatible with --model (multimodal models).")
@@ -169,8 +193,9 @@ def main(argv=None):
                         cosine_loss_alpha=hp["cosine_loss_alpha"], num_epochs=hp["num_epochs"],
                         data_augmentation=hp.get("data_augmentation", "burst_noise"))
     extended = args.training_mode != "default" and not args.unimodal_model
+    extra = {"evaluate": True} if args.evaluate else {}
     return experiment(config, model, Wrapper, model_name, scratch, data_dir, extended_data_module=extended, max_steps=args.max_steps,
-                      seeds=tuple(args.seeds))
+                      seeds=tuple(args.seeds), **extra)
 
 
 if __name__ == "__main__":

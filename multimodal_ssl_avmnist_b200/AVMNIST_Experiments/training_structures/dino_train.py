@@ -6,9 +6,10 @@ Differences that are documented, not hidden: the reference's legacy loop expects
 loop -- and unlike its Lightning path -- the teacher EMA runs AFTER the optimizer step.
 
 Downstream evaluation: `feature_extraction_loop` / `train_knn_classifier` (reference :327-369) run on the CUDA feature path +
-the device kNN kernels (SURVEY 8f-3); `train_downstream` / `compute_classification_metrics` (an MLP probe trained for 10 epochs +
-sklearn reports) stay outside the hot-path scope -- the per-epoch probe the checkpoint metric needs is
-`_DinoLightningBase.probe_accuracy` in models/dino.py."""
+the device kNN kernels (SURVEY 8f-3); `train_downstream` (the 10-epoch MLP probe on frozen features) runs on the device probe
+kernels (multimodal_ssl_avmnist_b200/probe.py, DESIGN.md section 4.11); `compute_classification_metrics` reduces a confusion
+matrix accumulated on the device to sklearn's classification_report; `compute_accuracies` is the post-training evaluation of
+the reference's run_dino.py:389 (kNN + MLP probe + metrics)."""
 import csv
 import json
 import os
@@ -105,9 +106,95 @@ def train_knn_classifier(pretrained_dino, train_dataloader, test_dataloader, n_n
     return knn, accuracy
 
 
-def _evaluation_out_of_scope(*a, **k):
-    raise NotImplementedError("the 10-epoch MLP probe / sklearn metric reports are outside the B200 hot-path scope (SURVEY 8f-3); "
-                              "see _DinoLightningBase.probe_accuracy for the per-epoch probe")
+def train_downstream(pretrained_model, train_loader, test_loader, num_epochs=10, learning_rate=1e-3, device="cuda", num_classes=10,
+                     is_dino_based=True, graph=True):
+    """The MLP probe of the frozen student (DESIGN.md section 4.11): a fresh DownstreamClassifier head (initial weights from the
+    global RNG), CrossEntropyLoss, AdamW(learning_rate) with torch's defaults, `num_epochs` epochs over train_loader with
+    train-mode features (batch statistics, fusion dropout, the probe's private copy of the running statistics), then an
+    evaluation of test_loader with eval-mode features after every epoch.  Every step runs on the device (probe.ProbeSession).
+    Returns (classifier, history): classifier is a DownstreamClassifier holding the trained head, so classifier(images,
+    spectrograms) works afterwards; history = {"train_loss", "val_loss", "val_acc" (%)} per epoch, losses per sample.
+    The reference's body of this function is not in this tree: the signature and the semantics follow its call site and
+    models/dino.py's DownstreamClassifier, not a pinned implementation."""
+    from models.dino import DownstreamClassifier
+    from multimodal_ssl_avmnist_b200.probe import ProbeSession
+    classifier = DownstreamClassifier(pretrained_model, num_classes=num_classes, is_dino_based=is_dino_based)
+    session = ProbeSession(pretrained_model, num_classes=num_classes, lr=learning_rate, weight_decay=1e-2, graph=graph,
+                           head=classifier.classifier)
+    classifier.encoder._probe = session.token            # classifier(...) evaluates with the probe's running statistics
+    history = {"train_loss": [], "val_loss": [], "val_acc": []}
+    for epoch in range(num_epochs):
+        for batch in train_loader:
+            session.train_batch(batch[0], batch[1], batch[2])
+        train_loss, _ = session.end_epoch()
+        ev = session.evaluate(test_loader)
+        history["train_loss"].append(train_loss)
+        history["val_loss"].append(ev["loss"])
+        history["val_acc"].append(100.0 * ev["accuracy"])
+        print(f"Epoch {epoch + 1}/{num_epochs}: train loss {train_loss:.4f}, val loss {ev['loss']:.4f}, val acc {100.0 * ev['accuracy']:.2f}%")
+    session.export_head()
+    classifier.to(pretrained_model.center.device).eval()
+    classifier.b200_probe = session
+    return classifier, history
 
 
-train_downstream = compute_classification_metrics = _evaluation_out_of_scope
+def metrics_from_confusion(cm):
+    """sklearn.metrics.classification_report(y_true, y_pred, output_dict=True, zero_division=0) from the confusion matrix
+    cm[label, pred] of those predictions (classes that neither occur nor are predicted are left out, as sklearn does), plus
+    "confusion_matrix" = cm as int64 [C, C]."""
+    import numpy as np
+    cm = np.asarray(cm, dtype=np.int64)
+    tp = np.diag(cm).astype(np.float64)
+    support = cm.sum(axis=1)
+    predicted = cm.sum(axis=0)
+    present = np.nonzero((support > 0) | (predicted > 0))[0]
+    out = {}
+    precision, recall, f1 = {}, {}, {}
+    for c in present:
+        precision[c] = tp[c] / predicted[c] if predicted[c] > 0 else 0.0
+        recall[c] = tp[c] / support[c] if support[c] > 0 else 0.0
+        den = 2 * tp[c] + (predicted[c] - tp[c]) + (support[c] - tp[c])
+        f1[c] = 2 * tp[c] / den if den > 0 else 0.0
+        out[str(int(c))] = {"precision": float(precision[c]), "recall": float(recall[c]), "f1-score": float(f1[c]),
+                            "support": float(support[c])}
+    total = float(support.sum())
+    out["accuracy"] = float(tp.sum() / total) if total > 0 else 0.0
+    for name, w in (("macro avg", np.ones(len(present))), ("weighted avg", support[present].astype(np.float64))):
+        ws = w.sum()
+        avg = lambda d: float(np.dot(w, [d[c] for c in present]) / ws) if ws > 0 else 0.0  # noqa: E731
+        out[name] = {"precision": avg(precision), "recall": avg(recall), "f1-score": avg(f1), "support": total}
+    out["confusion_matrix"] = cm
+    return out
+
+
+def compute_classification_metrics(classifier, loader, device="cuda", num_classes=10):
+    """Accuracy, per-class precision / recall / f1-score / support, macro and weighted averages (sklearn's
+    classification_report(output_dict=True, zero_division=0) definitions) and the int64 confusion matrix of a DownstreamClassifier
+    on `loader`.  Predictions and the confusion matrix are computed on the device (eval-mode features -> probe kernel); only the
+    [C, C] matrix comes back to the host."""
+    from multimodal_ssl_avmnist_b200.probe import ProbeSession
+    session = getattr(classifier, "b200_probe", None)
+    if session is None or session.C != num_classes:
+        fx = classifier.encoder
+        dino = fx._dino[0]
+        if fx._probe is None:
+            fx._probe = dino._b200.ensure(dino.center.device).begin_probe()
+        session = ProbeSession(dino, num_classes=num_classes, graph=False, head=classifier.classifier, probe=fx._probe)
+    else:
+        session.load_head(classifier.classifier)
+    return metrics_from_confusion(session.evaluate(loader)["confusion_matrix"])
+
+
+def compute_accuracies(pretrained_model, train_loader, test_loader, n_neighbors=5, num_epochs=10, learning_rate=1e-3, device="cuda",
+                       num_classes=10, is_dino_based=True):
+    """Post-training evaluation of a pretrained DINO model (reference run_dino.py:389): kNN accuracy of the frozen student's
+    features, the MLP probe (train_downstream) and its classification metrics on test_loader.
+    Returns {"knn_acc": %, "mlp_acc": %, "metrics": compute_classification_metrics(...)}."""
+    _, knn_acc = train_knn_classifier(pretrained_model, train_loader, test_loader, n_neighbors=n_neighbors, device=device,
+                                      is_dino_based=is_dino_based)
+    classifier, _ = train_downstream(pretrained_model, train_loader, test_loader, num_epochs=num_epochs, learning_rate=learning_rate,
+                                     device=device, num_classes=num_classes, is_dino_based=is_dino_based)
+    metrics = compute_classification_metrics(classifier, test_loader, device=device, num_classes=num_classes)
+    mlp_acc = 100.0 * metrics["accuracy"]
+    print(f"MLP Accuracy: {mlp_acc:.4f}%")
+    return {"knn_acc": float(knn_acc), "mlp_acc": mlp_acc, "metrics": metrics}

@@ -9,7 +9,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libavmnist_b200.so")
-SOURCES = ["core.cu", "loss.cu", "augment.cu", "encoder.cu", "linear.cu", "conv_tc.cu", "act8.cu", "gemm_tc.cu", "knn.cu", "dp.cu", "mix.cu"]  # missing files are skipped
+SOURCES = ["core.cu", "loss.cu", "augment.cu", "encoder.cu", "linear.cu", "conv_tc.cu", "act8.cu", "gemm_tc.cu", "knn.cu", "dp.cu", "mix.cu", "probe.cu"]  # missing files are skipped
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "-Xcompiler", "-fPIC",
               "--expt-relaxed-constexpr", "-Xptxas", "-v"]
 

@@ -99,16 +99,24 @@ __device__ __forceinline__ void adam_one(float& pi, float gi_raw, float& mi, flo
     pi = pi - step * (mi / denom);
 }
 
+// DECOUPLED (torch.optim.AdamW): p <- p * (1 - lr*wd) first, and no L2 term in the gradient; the rest is adam_one unchanged, so
+// with wd = 0 the update is bit-identical to Adam's.  `decay` is 1 - lr*wd rounded from double like torch's Python scalar (the
+// kernel recomputes it only when the learning rate comes from bc_dev).
+template <bool DECOUPLED>
 __global__ void __launch_bounds__(256) adam_flat_kernel(float* __restrict__ p, const float* __restrict__ g,
                                                         float* __restrict__ m, float* __restrict__ v, int64_t n, float lr,
                                                         float b1, float b2, float eps, float wd, float bc1, float bc2s,
-                                                        float gs, const float* __restrict__ bc_dev) {
+                                                        float gs, const float* __restrict__ bc_dev, float decay = 1.f) {
     const int64_t stride = (int64_t)gridDim.x * blockDim.x;
     if (bc_dev != nullptr) {          // CUDA-graph replay: the bias corrections (and the learning rate) of this step live on the device
         bc1 = __ldg(bc_dev);
         bc2s = __ldg(bc_dev + 1);
-        if (lr < 0.f) lr = __ldg(bc_dev + 2);
+        if (lr < 0.f) {
+            lr = __ldg(bc_dev + 2);
+            if (DECOUPLED) decay = (float)(1.0 - (double)lr * (double)wd);
+        }
     }
+    if (DECOUPLED) wd = 0.f;
     const float step = lr / bc1;
     // 128-bit accesses over the aligned body (the arenas are 16-byte aligned and padded; same arithmetic per element either way)
     const bool vec = ((reinterpret_cast<uintptr_t>(p) | reinterpret_cast<uintptr_t>(g) | reinterpret_cast<uintptr_t>(m) |
@@ -117,6 +125,12 @@ __global__ void __launch_bounds__(256) adam_flat_kernel(float* __restrict__ p, c
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += stride) {
         float4 pp = reinterpret_cast<float4*>(p)[i], mm = reinterpret_cast<float4*>(m)[i], vv = reinterpret_cast<float4*>(v)[i];
         const float4 gg = __ldg(reinterpret_cast<const float4*>(g) + i);
+        if (DECOUPLED) {
+            pp.x *= decay;
+            pp.y *= decay;
+            pp.z *= decay;
+            pp.w *= decay;
+        }
         adam_one(pp.x, gg.x, mm.x, vv.x, step, b1, b2, eps, wd, bc2s, gs);
         adam_one(pp.y, gg.y, mm.y, vv.y, step, b1, b2, eps, wd, bc2s, gs);
         adam_one(pp.z, gg.z, mm.z, vv.z, step, b1, b2, eps, wd, bc2s, gs);
@@ -127,6 +141,7 @@ __global__ void __launch_bounds__(256) adam_flat_kernel(float* __restrict__ p, c
     }
     for (int64_t i = n4 * 4 + (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
         float pi = p[i], mi = m[i], vi = v[i];
+        if (DECOUPLED) pi *= decay;
         adam_one(pi, __ldg(g + i), mi, vi, step, b1, b2, eps, wd, bc2s, gs);
         m[i] = mi;
         v[i] = vi;
@@ -240,7 +255,7 @@ int b200_adam_flat(float* param, const float* grad, float* exp_avg, float* exp_a
                    float beta2, float eps, float weight_decay, float bias_correction1, float bias_correction2_sqrt,
                    float grad_scale, void* stream) {
     B200_REQUIRE(param && grad && exp_avg && exp_avg_sq && n > 0, B200_E_ARG, "adam_flat: null pointer or n <= 0");
-    adam_flat_kernel<<<flat_grid(n, 4), 256, 0, as_stream(stream)>>>(param, grad, exp_avg, exp_avg_sq, n, lr, beta1, beta2,
+    adam_flat_kernel<false><<<flat_grid(n, 4), 256, 0, as_stream(stream)>>>(param, grad, exp_avg, exp_avg_sq, n, lr, beta1, beta2,
                                                                      eps, weight_decay, bias_correction1,
                                                                      bias_correction2_sqrt, grad_scale, nullptr);
     return launch_status("adam_flat");
@@ -255,9 +270,28 @@ int b200_adam_bias_dev(const int64_t* step_dev, double beta1, double beta2, floa
 int b200_adam_flat_dev(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, int64_t n, float lr, float beta1,
                        float beta2, float eps, float weight_decay, const float* bc_dev, float grad_scale, void* stream) {
     B200_REQUIRE(param && grad && exp_avg && exp_avg_sq && bc_dev && n > 0, B200_E_ARG, "adam_flat_dev: null pointer or n <= 0");
-    adam_flat_kernel<<<flat_grid(n, 4), 256, 0, as_stream(stream)>>>(param, grad, exp_avg, exp_avg_sq, n, lr, beta1, beta2,
+    adam_flat_kernel<false><<<flat_grid(n, 4), 256, 0, as_stream(stream)>>>(param, grad, exp_avg, exp_avg_sq, n, lr, beta1, beta2,
                                                                      eps, weight_decay, 1.f, 1.f, grad_scale, bc_dev);
     return launch_status("adam_flat_dev");
+}
+
+int b200_adamw_flat(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, int64_t n, float lr, float beta1,
+                    float beta2, float eps, float weight_decay, float bias_correction1, float bias_correction2_sqrt, void* stream) {
+    B200_REQUIRE(param && grad && exp_avg && exp_avg_sq && n > 0 && lr >= 0.f, B200_E_ARG, "adamw_flat: null pointer, n <= 0 or lr < 0");
+    const float decay = (float)(1.0 - (double)lr * (double)weight_decay);
+    adam_flat_kernel<true><<<flat_grid(n, 4), 256, 0, as_stream(stream)>>>(param, grad, exp_avg, exp_avg_sq, n, lr, beta1, beta2, eps,
+                                                                           weight_decay, bias_correction1, bias_correction2_sqrt, 1.f,
+                                                                           nullptr, decay);
+    return launch_status("adamw_flat");
+}
+
+int b200_adamw_flat_dev(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, int64_t n, float lr, float beta1,
+                        float beta2, float eps, float weight_decay, const float* bc_dev, void* stream) {
+    B200_REQUIRE(param && grad && exp_avg && exp_avg_sq && bc_dev && n > 0, B200_E_ARG, "adamw_flat_dev: null pointer or n <= 0");
+    const float decay = (float)(1.0 - (double)lr * (double)weight_decay);     // replaced on the device when lr < 0
+    adam_flat_kernel<true><<<flat_grid(n, 4), 256, 0, as_stream(stream)>>>(param, grad, exp_avg, exp_avg_sq, n, lr, beta1, beta2, eps,
+                                                                           weight_decay, 1.f, 1.f, 1.f, bc_dev, decay);
+    return launch_status("adamw_flat_dev");
 }
 
 int b200_counters_advance(int64_t* counters, int n, void* stream) {

@@ -1152,12 +1152,15 @@ class DinoStepEngine:
 
     @_main_chain
     @torch.no_grad()
-    def encode_features(self, images, audios=None, train=False, teacher=False, probe=None):
+    def encode_features(self, images, audios=None, train=False, teacher=False, probe=None, step_dev=None):
         """Encoder features [B, O] of an UN-augmented batch (images [B,28,28] fp32 in [0,1] or uint8, audios [B,112,112] fp32 in
         [0,1] or uint8), as DownstreamClassifier / FeatureExtractor of the reference use them (models/dino.py:1764-1850).
         train=False: BatchNorm with running statistics, no dropout (module.eval()); train=True: batch statistics and an active
         fusion dropout.  probe (a begin_probe() token): the running statistics read / updated are the probe copy's, and every
-        train-mode call draws a fresh dropout mask; without a token train-mode updates go to scratch and eval reads the live ones."""
+        train-mode call draws a fresh dropout mask; without a token train-mode updates go to scratch and eval reads the live ones.
+        step_dev (int64 device scalar, with a token): the probe's dropout position is read from it instead of the token's host
+        counter -- the same mask stream, (rng_step + *step_dev) * 4 + 3 -- so a captured CUDA graph draws a fresh mask per replay;
+        the caller advances it."""
         B = self._batch_size(images, audios)
         w = self._eval_workspace(B)
         P = self.T if teacher else self.S
@@ -1185,7 +1188,10 @@ class DinoStepEngine:
             fmask = w["e.fmask"]
             if probe is not None:
                 probe["step"] += 1
-            ops.dropout_mask(fmask, self.fusion_dropout, self.seed + 17, (self.rng_step + (probe["step"] if probe is not None else 0)) * 4 + 3)
+            if step_dev is not None:
+                ops.dropout_mask(fmask, self.fusion_dropout, self.seed + 17, self.rng_step * 4 + 3, step_dev=step_dev)
+            else:
+                ops.dropout_mask(fmask, self.fusion_dropout, self.seed + 17, (self.rng_step + (probe["step"] if probe is not None else 0)) * 4 + 3)
         self._eval_wrole = "t" if teacher else "s"
         return self._encode(w, "e", P, bns, xi, xa, B, B, B, fmask, train=train)
 

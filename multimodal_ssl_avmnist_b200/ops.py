@@ -98,6 +98,20 @@ def adam_flat_dev(param, grad, exp_avg, exp_avg_sq, bc_dev, lr, beta1=0.9, beta2
                                           lr, beta1, beta2, eps, weight_decay, _ptr(bc_dev, F32), grad_scale, _stream()), "adam_flat")
 
 
+def adamw_flat(param, grad, exp_avg, exp_avg_sq, step, lr, beta1=0.9, beta2=0.999, eps=1e-8, weight_decay=1e-2):
+    """torch.optim.AdamW step `step` (1-based): p *= 1 - lr*weight_decay, then the Adam update without an L2 term."""
+    bc1 = 1 - beta1 ** step
+    bc2s = (1 - beta2 ** step) ** 0.5
+    _lib.check(_lib_().b200_adamw_flat(_ptr(param, F32), _ptr(grad, F32), _ptr(exp_avg, F32), _ptr(exp_avg_sq, F32), param.numel(),
+                                       lr, beta1, beta2, eps, weight_decay, bc1, bc2s, _stream()), "adamw_flat")
+
+
+def adamw_flat_dev(param, grad, exp_avg, exp_avg_sq, bc_dev, lr, beta1=0.9, beta2=0.999, eps=1e-8, weight_decay=1e-2):
+    """adamw_flat with the bias corrections read from bc_dev (written by adam_bias_dev; CUDA-graph replay)."""
+    _lib.check(_lib_().b200_adamw_flat_dev(_ptr(param, F32), _ptr(grad, F32), _ptr(exp_avg, F32), _ptr(exp_avg_sq, F32), param.numel(),
+                                           lr, beta1, beta2, eps, weight_decay, _ptr(bc_dev, F32), _stream()), "adamw_flat_dev")
+
+
 def counters_advance(counters):
     _lib.check(_lib_().b200_counters_advance(_ptr(counters, I64), counters.numel(), _stream()), "counters_advance")
 
@@ -643,10 +657,29 @@ def knn_predict(train_feats, train_labels, test_feats, k=5, n_classes=10, return
     return (pred, nbr) if return_neighbours else pred
 
 
+# ---- downstream MLP probe (train_downstream; csrc/probe.cu) -------------------------------------------------------------
+def probe_work_floats(B, C):
+    n = int(_lib_().b200_probe_work_floats(B, C))
+    if n < 0:
+        raise _lib.B200Error(f"probe_work_floats: unsupported shape B={B} C={C}")
+    return n
+
+
+def probe_mlp_fwd_bwd(x, w1, b1, w2, b2, labels, work, loss_sum, correct, grad=None, preds=None, confusion=None, train=True):
+    """DownstreamClassifier head + CrossEntropyLoss on features x [B, O]: train=True writes [dW1 | db1 | dW2 | db2] into grad;
+    train=False writes the argmax into preds [B] and counts [label, pred] into confusion [C, C] (both optional).  Always:
+    loss_sum (fp64 [1]) += the batch's loss sum, correct (int64 [1]) += its correct predictions."""
+    B, O = x.shape
+    C = b2.numel()
+    _lib.check(_lib_().b200_probe_mlp_fwd_bwd(_ptr(x, F32), _ptr(w1, F32), _ptr(b1, F32), _ptr(w2, F32), _ptr(b2, F32), _ptr(labels, I64),
+                                              B, O, C, int(bool(train)), _ptr(grad, F32), _ptr(work, F32), _ptr(loss_sum, F64),
+                                              _ptr(correct, I64), _ptr(preds, I64), _ptr(confusion, I64), _stream()), "probe_mlp_fwd_bwd")
+
+
 # ---- launch accounting and optional per-op timing ------------------------------------------------------------
 # Every wrapper above issues a fixed number of kernel launches; the table lists the ones that issue more than one.
-_LAUNCHES = {"gate_grad": 2, "ntxent_fwd_bwd": 5, "conv_tc_wgrad_l0_fused": 3, "conv_tc_wgrad": 2, "conv_bwd_weight": 3, "linear_bwd_weight": 3, "infonce_fwd_bwd": 9}
-_NOT_KERNELS = {"conv_tc_wgrad_variant", "gate_grad_work_floats", "knn_predict", "conv_tc_pool_supported", "conv_tc_dgrad_bnstat_supported", "quad8_width", "ntxent_work_floats", "conv_tc_wgrad_l0_fused_work_floats", "conv_tc_wgrad_work_floats", "conv_tc_supported", "conv_tc_weight_bytes", "dino_loss_parts", "infonce_work_floats", "conv_supported", "conv_bwd_weight_work_floats", "launch_count", "start_profile", "stop_profile"}
+_LAUNCHES = {"gate_grad": 2, "probe_mlp_fwd_bwd": 2, "ntxent_fwd_bwd": 5, "conv_tc_wgrad_l0_fused": 3, "conv_tc_wgrad": 2, "conv_bwd_weight": 3, "linear_bwd_weight": 3, "infonce_fwd_bwd": 9}
+_NOT_KERNELS = {"conv_tc_wgrad_variant", "probe_work_floats", "gate_grad_work_floats", "knn_predict", "conv_tc_pool_supported", "conv_tc_dgrad_bnstat_supported", "quad8_width", "ntxent_work_floats", "conv_tc_wgrad_l0_fused_work_floats", "conv_tc_wgrad_work_floats", "conv_tc_supported", "conv_tc_weight_bytes", "dino_loss_parts", "infonce_work_floats", "conv_supported", "conv_bwd_weight_work_floats", "launch_count", "start_profile", "stop_profile"}
 LAUNCH_COUNT = 0
 _PROFILE = None          # None, or a list receiving (name, start_event, end_event, meta)
 
