@@ -20,7 +20,7 @@ import torch
 
 from . import dp
 from . import ops
-from .engine import F32, Arena, DinoStepEngine, _BN, _conv, _lin, _vec2, head_params
+from .engine import F32, Arena, DinoStepEngine, _BN, _conv, _lin, _vec2, _zero_arena, head_params
 
 IMG_LAYERS = [("image_encoder.encoder.0", "image_encoder.encoder.1", 1, 32, 28, 3, 1), ("image_encoder.encoder.4", "image_encoder.encoder.5", 32, 64, 14, 3, 1),
               ("image_encoder.encoder.8", "image_encoder.encoder.9", 64, 128, 7, 3, 1)]
@@ -48,7 +48,7 @@ def contrastive_params(O, P):
 
 class ContrastiveStepEngine(DinoStepEngine):
     def __init__(self, kind="infonce", output_dim=256, projection_dim=256, learning_rate=1e-4, temperature=0.07, seed=0, device=None,
-                 precision="bf16", fused_pool=False, process_group=None, data_parallel=None, mode_seed=0):
+                 precision="bf16", process_group=None, data_parallel=None, mode_seed=0):
         if not torch.cuda.is_available():
             raise ops._lib.B200Error("ContrastiveStepEngine needs a CUDA device: the hot path has no CPU fallback")
         ops._lib.load()
@@ -80,33 +80,17 @@ class ContrastiveStepEngine(DinoStepEngine):
             self.bn_s["enc." + bn] = _BN(co, self.device)
         for m in ("image", "audio"):
             self.bn_s[f"enc.{m}_projection_head.mlp.1"] = _BN(512, self.device)
-        self.tc = {}
-        for mod, layers in (("img", IMG_LAYERS), ("aud", AUD_LAYERS)):
-            self.tc[mod] = [precision == "bf16" and ops.conv_tc_supported(ci, co, hw, hw, k, pad) and
-                            (ci == 1 or ops.conv_tc_supported(co, ci, hw + 2 * pad - k + 1, hw + 2 * pad - k + 1, k, k - 1 - pad))
-                            for (conv, bn, ci, co, hw, k, pad) in layers]
+        self._select_tc_layers(("s",))
         # no max-pool in the forward epilogues: for these 32 - 256 channel layers the fused variant measured slower than conv + pool pass
-        # (engine.py, profiles/r2zf_*); `fused_pool=True` re-enables it on the 112x112 first audio layer for A/B runs
-        self.fused_pool = bool(fused_pool)
-        self.pool = {"s": {mod: [self.fused_pool and bool(self.tc[mod][li]) and ops.conv_tc_pool_supported(ci, co, hw, hw, k, pad) and ci == 1 and hw >= 112
-                                 for li, (conv, bn, ci, co, hw, k, pad) in enumerate(layers)] for mod, layers in (("img", IMG_LAYERS), ("aud", AUD_LAYERS))}}
-        self.pool["t"] = self.pool["s"]
+        # (engine.py, profiles/r2zf_*)
+        self.fused_pool = False
+        self.pool = {r: {mod: [False] * len(layers) for mod, layers in (("img", IMG_LAYERS), ("aud", AUD_LAYERS))} for r in ("s", "t")}
         self.fused_bnstat = False
         self.bnstat = {mod: [False] * len(layers) for mod, layers in (("img", IMG_LAYERS), ("aud", AUD_LAYERS))}
-        self._tcw, self._prep_desc = {}, {}
-        for mod, layers in (("img", IMG_LAYERS), ("aud", AUD_LAYERS)):
-            for li, (conv, bn, ci, co, hw, k, pad) in enumerate(layers):
-                if self.tc[mod][li]:
-                    self._tcw[("s", mod, li)] = torch.empty(ops.conv_tc_weight_bytes(ci, co, k), dtype=torch.uint8, device=self.device)
-                    if ci > 1:
-                        self._tcw[("flip", mod, li)] = torch.empty(ops.conv_tc_weight_bytes(co, ci, k), dtype=torch.uint8, device=self.device)
         self.overlap_teacher = True
-        self.stream_priorities, self._main_stream = False, None
-        self._side_stream = torch.cuda.Stream(device=self.device)
         self._lin_wg_stream = torch.cuda.Stream(device=self.device)
         self._lin_wg_pending = False
         self._wgrad_streams = {m: torch.cuda.Stream(device=self.device) for m in ("img", "aud")}
-        self._eval_wrole = "s"
         self._ws = {}
         # host draw of the SimCLR modality pairing (torch.randint in the reference): the SAME sequence on every rank (mode_seed, not the
         # per-rank seed), so that all ranks run -- and exchange -- the same branches
@@ -154,61 +138,16 @@ class ContrastiveStepEngine(DinoStepEngine):
         """Buffers for up to two encoder calls per modality; _combo() hands out the prefix views of a (calls_img, calls_aud) schedule."""
         if B in self._ws:
             return self._ws[B]
-        dev, BF = self.device, torch.bfloat16
+        dev = self.device
 
         def e(*shape, dtype=F32):
             return torch.empty(*shape, dtype=dtype, device=dev)
 
         w = {"B": B}
-        zarena = torch.zeros(1 << 16, dtype=torch.float64, device=dev)
-        zoff = [0]
-
-        def zalloc(*shape):
-            n = int(math.prod(shape))
-            o = zoff[0]
-            zoff[0] = o + (n + 1) // 2 * 2
-            if zoff[0] > zarena.numel():
-                raise ops._lib.B200Error("zero arena too small")
-            return zarena[o:o + n].view(*shape)
-
-        w["zarena"] = zarena
+        w["zarena"], zalloc = _zero_arena(1 << 16, dev)
         N = 2 * B
         w["x_img"], w["x_aud"] = e(N, 1, 28, 28), e(N, 1, 112, 112)
-        for mod, layers in (("img", IMG_LAYERS), ("aud", AUD_LAYERS)):
-            sc = dict(wg=0, z=0, p=0, z8=0)
-            for li, (conv, bn, ci, co, hw, k, pad) in enumerate(layers):
-                ho = hw + 2 * pad - k + 1
-                tc = self.tc[mod][li]
-                next_tc = li + 1 < len(layers) and self.tc[mod][li + 1]
-                if tc and ci == 1:
-                    w[f"{mod}.xs8"] = e(N, hw, ops.quad8_width(hw, pad), 8, dtype=BF)
-                if tc and self.pool["s"][mod][li]:
-                    w[f"s.{mod}.e{li}"] = e(N, co // 8, ho // 2, ho // 2, 8, dtype=torch.float16)
-                w[f"s.{mod}.z{li}"] = e(N, co // 8, ho, ho, 8, dtype=torch.float16) if tc else e(N, co, ho, ho)
-                if next_tc:
-                    w[f"s.{mod}.p8{li}"] = e(N, co // 8, ho // 2, ho // 2, 8, dtype=BF)
-                if not next_tc or not tc:
-                    w[f"s.{mod}.p{li}"] = e(N, co, ho // 2, ho // 2)
-                w[f"s.{mod}.stats{li}"] = zalloc(2, co, 2)
-                w[f"s.{mod}.sums{li}"] = zalloc(2, co, 2)
-                for nm in ("scale", "shift", "mean", "invstd"):
-                    w[f"s.{mod}.{nm}{li}"] = e(2, co)
-                if tc:
-                    sc["wg"] = max(sc["wg"], ops.conv_tc_wgrad_work_floats(N, ci, co, hw, hw, k, pad))
-                    if ci == 1:
-                        sc["wg"] = max(sc["wg"], ops.conv_tc_wgrad_l0_fused_work_floats(N, B, co, hw, hw, k, pad))
-                    else:
-                        sc["z8"] = max(sc["z8"], N * co * ho * ho)
-                else:
-                    sc["wg"] = max(sc["wg"], ops.conv_bwd_weight_work_floats(N, ci, co, hw, hw, k, pad))
-                    sc["z"] = max(sc["z"], N * co * ho * ho)
-                sc["p"] = max(sc["p"], N * co * (ho // 2) * (ho // 2), N * ci * hw * hw if li > 0 else 0)
-            w[f"{mod}.dz"] = e(max(sc["z"], 4))
-            w[f"{mod}.dz8"] = e(max(sc["z8"], 8), dtype=BF)
-            w[f"{mod}.dz8b"] = e(max(sc["z8"], 8), dtype=BF)
-            w[f"{mod}.dbsum"] = zalloc(8, 256)
-            w[f"{mod}.dp_a"], w[f"{mod}.dp_b"] = e(sc["p"]), e(sc["p"])
-            w[f"{mod}.wg_work"], w[f"{mod}.wg_work_b"] = e(max(sc["wg"], 4)), e(max(sc["wg"], 4))
+        self._stack_buffers(w, "s", N, B, e, zalloc)
         O, P = self.O, self.P
         w["img.gap"], w["img.e14"], w["aud.gap"] = e(N, 128), e(N, 512), e(N, 256)
         w["d.img.gap"], w["d.img.e14"], w["d.aud.gap"] = e(N, 128), e(N, 512), e(N, 256)

@@ -29,7 +29,6 @@ import contextlib
 import math
 
 import numpy as np
-import os
 
 import torch
 
@@ -219,15 +218,21 @@ def _rows(x, n):
     return None if x is None else x[:n]
 
 
-def _main_chain(fn):
-    """Method decorator: the launches of `fn` go to the engine's high-priority main stream (DinoStepEngine._on_main)."""
-    import functools
+def _zero_arena(n, device):
+    """Every accumulator of a workspace that must be zero when a step starts (BatchNorm statistics, backward sums, bias-gradient
+    sums) lives in ONE float64 arena of n doubles: one memset per step instead of two dozen.  Returns (arena, zalloc), where
+    zalloc(*shape) hands out the next 16-byte aligned view."""
+    arena = torch.zeros(n, dtype=torch.float64, device=device)
+    end = 0
 
-    @functools.wraps(fn)
-    def wrapped(self, *args, **kwargs):
-        with self._on_main():
-            return fn(self, *args, **kwargs)
-    return wrapped
+    def zalloc(*shape):
+        nonlocal end
+        k = int(math.prod(shape))
+        o, end = end, end + (k + 1) // 2 * 2
+        if end > arena.numel():
+            raise ops._lib.B200Error("zero arena too small")
+        return arena[o:o + k].view(*shape)
+    return arena, zalloc
 
 
 class DinoStepEngine:
@@ -242,7 +247,7 @@ class DinoStepEngine:
                  n_global_views=2, n_local_views=4, momentum=0.996, center_momentum=0.9, student_temperature=0.1,
                  teacher_temperature=0.04, learning_rate=1e-4, weight_decay=1e-6, dropout=0.3, fusion_dropout=0.3, alpha=1.0,
                  cosine_loss_alpha=0.0, augment_values=None, seed=0, device=None, process_group=None, data_parallel=None,
-                 precision="bf16", fused_pool=True, fused_bnstat=False, stream_priorities=False):
+                 precision="bf16", fused_pool=True, fused_bnstat=False):
         if not torch.cuda.is_available():
             raise ops._lib.B200Error("DinoStepEngine needs a CUDA device: the hot path has no CPU fallback")
         ops._lib.load()
@@ -315,10 +320,6 @@ class DinoStepEngine:
         self.n_trainable_prefix = self.student.range_of([n for n, _ in enc_used + head])[1]
         self.aux_range = self.student.range_of([n for n, _ in aux]) if aux else None
         self.grad_plan = dp.GradientPlan([(0, self.n_trainable_prefix)] + ([self.aux_range] if self.aux_range else []))
-        # gradient exchange in two slices: [split, end of the trainable prefix) -- audio encoder linear, fusion MLP, projection head:
-        # complete as soon as the linear weight gradients are (early in the backward pass), exchanged beside the conv stacks'
-        # backward -- and [0, split): the conv stacks + the image encoder linear, complete at the end of the backward pass
-        self._bucket_split = self.student.offsets[self.top["aud"][2] + ".weight"][0] if self.multi else 0
         self._grad_scale = 1.0
         self.grad = torch.zeros_like(self.student.flat)
         self.exp_avg = torch.zeros_like(self.student.flat)
@@ -335,17 +336,7 @@ class DinoStepEngine:
         for m in ("aux_image", "aux_audio"):
             if aux:
                 self.bn_s[f"{m}.mlp.1"] = _BN(512, self.device)
-        # tensor-core layers (tcgen05, bf16 act8 activations, fp32 accumulate): every C_in >= 8 convolution the library supports
-        self.tc = {}
-        for mod, layers in (("img", self.img_layers), ("aud", self.aud_layers)):
-            self.tc[mod] = [precision == "bf16" and ops.conv_tc_supported(ci, co, hw, hw, k, pad) and
-                            (ci == 1 or ops.conv_tc_supported(co, ci, hw + 2 * pad - k + 1, hw + 2 * pad - k + 1, k, k - 1 - pad))
-                            for (conv, bn, ci, co, hw, k, pad) in layers]
-        for mod in self.tc:
-            # a tensor-core first layer runs its backward fused into the weight-gradient kernel (dz stays in shared memory),
-            # which consumes the bf16 act8 pooled gradient written by the second layer's tensor-core data gradient
-            if self.tc[mod] and self.tc[mod][0] and not (len(self.tc[mod]) > 1 and self.tc[mod][1]):
-                self.tc[mod][0] = False
+        self._select_tc_layers(("s", "t"))
         # forward layers whose 2x2 max-pool runs inside the convolution's epilogue (the pooled extreme e, a quarter of z, goes to the
         # BatchNorm-apply kernel).  The epilogue pays for it with a per-tile barrier between its four warps (profiles/r2e_*): it wins
         # where no z is written at all (teacher, evaluation) and on the HBM-bound first audio layer of the student; the student's other
@@ -370,47 +361,18 @@ class DinoStepEngine:
                              ops.conv_tc_dgrad_bnstat_supported(co, ci, hw + 2 * pad - k + 1, hw + 2 * pad - k + 1, k, k - 1 - pad)
                              for li, (conv, bn, ci, co, hw, k, pad) in enumerate(layers)]
                        for mod, layers in (("img", self.img_layers), ("aud", self.aud_layers))}
-        self._tcw = {}
-        self._prep_desc = {}
-        for mod, layers in (("img", self.img_layers), ("aud", self.aud_layers)):
-            for li, (conv, bn, ci, co, hw, k, pad) in enumerate(layers):
-                if self.tc[mod][li]:
-                    for role in ("s", "t"):
-                        self._tcw[(role, mod, li)] = torch.empty(ops.conv_tc_weight_bytes(ci, co, k), dtype=torch.uint8, device=self.device)
-                    if ci > 1:
-                        self._tcw[("flip", mod, li)] = torch.empty(ops.conv_tc_weight_bytes(co, ci, k), dtype=torch.uint8, device=self.device)
         self.overlap_teacher = True
-        # Stream priorities (optional, `stream_priorities=True`).  Most conv kernels are persistent grids that fill the GPU, so with several
-        # streams in flight every SM slot is taken and hundreds of CTAs are pending; a one-CTA kernel of the main chain (bn_finalize, bias /
-        # BatchNorm parameter gradients) then waits 0.15 - 0.25 ms for a slot behind them (event timeline, tools/timeline_step.py,
-        # profiles/r2t_timeline_*.txt).  With the main chain on a high-priority stream (teacher / image stack below it, weight gradients
-        # and the augmentation prefetch at the bottom) the block scheduler serves its pending CTAs first and the main chain of a B = 1024
-        # step ends 0.77 ms earlier -- but the step does NOT get shorter (7.65 vs 7.62 ms): the side streams' work then forms a 1.2 ms
-        # tail.  The step is bound by the total work of its kernels on a saturated GPU, not by the latency of its critical chain.
-        lo, hi = 0, -1
-        try:
-            hi = int(os.environ.get("B200_TOP_PRIORITY", "-3"))
-        except ValueError:
-            pass
-        self.stream_priorities = bool(stream_priorities)
-
-        def mk(level):          # level 0 = top ... 3 = bottom; clamped by the driver to the device's priority range
-            return torch.cuda.Stream(device=self.device, priority=(min(lo, hi + level) if self.stream_priorities else 0))
-
-        self._main_stream = mk(0) if self.stream_priorities else None
-        self._side_stream = mk(1)
-        self._lin_wg_stream = mk(3)       # linear weight gradients
+        # all streams at the default priority: a high-priority main chain ends earlier but does not shorten the step, which is bound
+        # by the total work of its kernels on a saturated GPU (DESIGN.md, "What the step is bound by")
+        self._side_stream = torch.cuda.Stream(device=self.device)
+        self._lin_wg_stream = torch.cuda.Stream(device=self.device)       # linear weight gradients
         self._lin_wg_pending = False
-        self._side_stream2 = mk(1)
-        self._wgrad_streams = {m: mk(2) for m in ("img", "aud")}
-        self._aug_stream = mk(3)
+        self._side_stream2 = torch.cuda.Stream(device=self.device)
+        self._wgrad_streams = {m: torch.cuda.Stream(device=self.device) for m in ("img", "aud")}
+        self._aug_stream = torch.cuda.Stream(device=self.device)
         # data parallel: the exchange runs inside the C ABI (NCCL, b200_dp_*) on a communication stream beside the compute streams
         self.comm = dp.AbiComm.get(process_group) if self.world > 1 else None
         self._comm_stream = torch.cuda.Stream(device=self.device) if self.world > 1 else None
-        # exchange the late-layout gradient slice beside the conv stacks' backward?  Measured at N = 2 (profiles/r2c_*): the NCCL CTAs
-        # take SMs from the persistent conv kernels (grids sized to fill the GPU) and the step gets 0.13 ms SLOWER, so the default
-        # is one exchange at the end of the backward pass (it still overlaps the teacher EMA)
-        self.overlap_grad_exchange = False
         self._center_ready = None          # event: the all-reduced centre EMA of the last step has landed
         self._comm_pending = False         # gradient all-reduces in flight on the communication stream
         self._prefetch, self._step_done, self._step_done_prev = None, None, None
@@ -419,19 +381,26 @@ class DinoStepEngine:
         self._init_parameters()
         self.set_augmentation(augment_values)
 
-    @contextlib.contextmanager
-    def _on_main(self):
-        """Run the enclosed launches on the engine's high-priority main stream, ordered after the caller's current stream, and make the
-        caller's stream wait for them afterwards (a no-op when priorities are off or we already are on that stream)."""
-        hp = self._main_stream
-        cur = torch.cuda.current_stream()
-        if hp is None or cur == hp:
-            yield
-            return
-        hp.wait_stream(cur)
-        with torch.cuda.stream(hp):
-            yield
-        cur.wait_stream(hp)
+    def _select_tc_layers(self, roles):
+        """self.tc[mod][li]: does conv layer li of a stack run on the tensor cores (tcgen05, bf16 act8 activations, fp32 accumulate)?
+        Every convolution whose forward and (for C_in > 1) flipped data gradient the library supports, on the bf16 path.  Allocates
+        the bf16 weight images of those layers for each role in `roles` and, for C_in > 1, the flipped image of the data gradient."""
+        self.tc, self._tcw, self._prep_desc = {}, {}, {}
+        for mod, layers in (("img", self.img_layers), ("aud", self.aud_layers)):
+            tc = [self.precision == "bf16" and ops.conv_tc_supported(ci, co, hw, hw, k, pad) and
+                  (ci == 1 or ops.conv_tc_supported(co, ci, hw + 2 * pad - k + 1, hw + 2 * pad - k + 1, k, k - 1 - pad))
+                  for (conv, bn, ci, co, hw, k, pad) in layers]
+            # a tensor-core first layer runs its backward fused into the weight-gradient kernel (dz stays in shared memory),
+            # which consumes the bf16 act8 pooled gradient written by the second layer's tensor-core data gradient
+            if tc and tc[0] and not (len(tc) > 1 and tc[1]):
+                tc[0] = False
+            self.tc[mod] = tc
+            for li, (conv, bn, ci, co, hw, k, pad) in enumerate(layers):
+                if tc[li]:
+                    for role in roles:
+                        self._tcw[(role, mod, li)] = torch.empty(ops.conv_tc_weight_bytes(ci, co, k), dtype=torch.uint8, device=self.device)
+                    if ci > 1:
+                        self._tcw[("flip", mod, li)] = torch.empty(ops.conv_tc_weight_bytes(co, ci, k), dtype=torch.uint8, device=self.device)
 
     # ------------------------------------------------------------------------------------------------------
     def _init_parameters(self):
@@ -497,20 +466,7 @@ class DinoStepEngine:
             return torch.empty(*shape, dtype=dtype, device=dev)
 
         w = {"B": B, "Ns": Ns, "Nt": Nt}
-        # every accumulator that must be zero when a step starts (BatchNorm statistics, backward sums, bias-gradient sums)
-        # lives in ONE float64 arena: one memset per step instead of two dozen
-        zarena = torch.zeros(1 << 17, dtype=torch.float64, device=dev)
-        zoff = [0]
-
-        def zalloc(*shape):
-            n = int(math.prod(shape))
-            o = zoff[0]
-            zoff[0] = o + (n + 1) // 2 * 2
-            if zoff[0] > zarena.numel():
-                raise ops._lib.B200Error("zero arena too small")
-            return zarena[o:o + n].view(*shape)
-
-        w["zarena"] = zarena
+        w["zarena"], zalloc = _zero_arena(1 << 17, dev)
         # augmentation (the sampler always draws the audio records; the image records only when there is an image stack)
         if self.img_layers:
             w["img_ops"] = torch.zeros(B, V, A.MAX_OPS, A.OP_WORDS, dtype=torch.int32, device=dev)
@@ -523,57 +479,11 @@ class DinoStepEngine:
             w["x_img"] = e(Ns, 1, 28, 28)
         if self.aud_layers:
             w["x_aud"] = e(Ns, 1, 112, 112)
-        scr = {m: dict(wg=0, z=0, p=0, z8=0) for m in ("img", "aud")}       # backward scratch sizes per modality stack
-        BF = torch.bfloat16
-        for role, N in (("s", Ns), ("t", Nt)):
-            for mod, layers in (("img", self.img_layers), ("aud", self.aud_layers)):
-                for li, (conv, bn, ci, co, hw, k, pad) in enumerate(layers):
-                    ho = hw + 2 * pad - k + 1
-                    nv = N // B
-                    tc = self.tc[mod][li]
-                    next_tc = li + 1 < len(layers) and self.tc[mod][li + 1]
-                    if tc and ci == 1 and role == "s":
-                        wq = ops.quad8_width(hw, pad)
-                        w[f"{mod}.xs8"] = e(N, hw, wq, 8, dtype=BF)             # first-layer input, quad8 (shared by the teacher)
-                        w[f"{mod}.xs8_b"] = e(N, hw, wq, 8, dtype=BF)           # ... and the slot the next step's views are prefetched into
-                    pooled = tc and self.pool[role][mod][li]
-                    if pooled:
-                        w[f"{role}.{mod}.e{li}"] = e(N, co // 8, ho // 2, ho // 2, 8, dtype=torch.float16)     # 2x2 window extreme of z
-                    if tc and (role == "s" or not pooled):
-                        w[f"{role}.{mod}.z{li}"] = e(N, co // 8, ho, ho, 8, dtype=torch.float16)   # act8 layout, fp16: never an MMA operand
-                    elif not tc:
-                        w[f"{role}.{mod}.z{li}"] = e(N, co, ho, ho)
-                    if next_tc:
-                        w[f"{role}.{mod}.p8{li}"] = e(N, co // 8, ho // 2, ho // 2, 8, dtype=BF)
-                    if not next_tc or not tc:
-                        w[f"{role}.{mod}.p{li}"] = e(N, co, ho // 2, ho // 2)
-                    w[f"{role}.{mod}.stats{li}"] = zalloc(nv, co, 2)
-                    for nm in ("scale", "shift", "mean", "invstd"):
-                        w[f"{role}.{mod}.{nm}{li}"] = e(nv, co)
-                    if role == "s":
-                        w[f"s.{mod}.sums{li}"] = zalloc(nv, co, 2)
-                        sc = scr[mod]
-                        if tc:
-                            sc["wg"] = max(sc["wg"], ops.conv_tc_wgrad_work_floats(N, ci, co, hw, hw, k, pad))
-                            if ci == 1:
-                                # fused apply + weight gradient: this layer's dz never exists in HBM
-                                sc["wg"] = max(sc["wg"], ops.conv_tc_wgrad_l0_fused_work_floats(N, B, co, hw, hw, k, pad))
-                            else:
-                                sc["z8"] = max(sc["z8"], N * co * ho * ho)
-                        else:
-                            sc["wg"] = max(sc["wg"], ops.conv_bwd_weight_work_floats(N, ci, co, hw, hw, k, pad))
-                            sc["z"] = max(sc["z"], N * co * ho * ho)
-                        sc["p"] = max(sc["p"], N * co * (ho // 2) * (ho // 2), N * ci * hw * hw if li > 0 else 0)
-        for m, sc in scr.items():           # one scratch set per stack: the two stacks' backward passes run on different streams
-            if sc["p"] == 0:
-                continue
-            w[f"{m}.dz"] = e(max(sc["z"], 4))
-            w[f"{m}.dz8"] = e(max(sc["z8"], 8), dtype=BF)
-            w[f"{m}.dz8b"] = e(max(sc["z8"], 8), dtype=BF)      # second buffer: the weight gradient of layer l overlaps layer l-1
-            w[f"{m}.dbsum"] = zalloc(8, 256)
-            w[f"{m}.dp_a"], w[f"{m}.dp_b"] = e(sc["p"]), e(sc["p"])
-            w[f"{m}.wg_work"] = e(max(sc["wg"], 4))
-            w[f"{m}.wg_work_b"] = e(max(sc["wg"], 4))
+        self._stack_buffers(w, "s", Ns, B, e, zalloc)
+        self._stack_buffers(w, "t", Nt, B, e, zalloc)
+        for m in ("img", "aud"):             # the spare first-layer input that prefetch_augment fills with the next step's views
+            if f"{m}.xs8" in w:
+                w[f"{m}.xs8_b"] = torch.empty_like(w[f"{m}.xs8"])
         E, O, P = self.E, self.O, self.P
         Nv = V * B
         if self.multi:
@@ -635,6 +545,62 @@ class DinoStepEngine:
             w["d.emb"] = e(Nv, O)          # cosine-consistency gradient (UniModalDINO, cosine_loss_alpha may be switched on later)
         self._ws[B] = w
         return w
+
+    def _stack_buffers(self, w, role, N, B, e, zalloc):
+        """The buffers both conv stacks need for one role ('s' student, 't' teacher, 'e' evaluation; 'e' follows the teacher's
+        pool table) on N = views * B samples.  Per layer: the pooled window extreme e where the forward pools in the conv epilogue,
+        the conv output z (unless a pooled layer of a role without backward), the pooled activation (act8 p8 when the next layer
+        reads it on the tensor cores, fp32 NCHW p otherwise), the BatchNorm statistics (zalloc, per view-call) and the affine /
+        normalisation vectors.  Roles 's' and 'e' also get the first-layer quad8 input xs8 (the teacher reads a prefix of the
+        student's); the student gets the backward sums and one backward scratch set per stack (the two stacks' backward passes
+        run on different streams)."""
+        BF = torch.bfloat16
+        nv = N // B
+        pool = self.pool["s" if role == "s" else "t"]
+        for mod, layers in (("img", self.img_layers), ("aud", self.aud_layers)):
+            sc = dict(wg=0, z=0, p=0, z8=0)
+            for li, (conv, bn, ci, co, hw, k, pad) in enumerate(layers):
+                ho = hw + 2 * pad - k + 1
+                tc = self.tc[mod][li]
+                next_tc = li + 1 < len(layers) and self.tc[mod][li + 1]
+                if tc and ci == 1 and role != "t":
+                    w[f"{mod}.xs8"] = e(N, hw, ops.quad8_width(hw, pad), 8, dtype=BF)
+                pooled = tc and pool[mod][li]
+                if pooled:
+                    w[f"{role}.{mod}.e{li}"] = e(N, co // 8, ho // 2, ho // 2, 8, dtype=torch.float16)     # 2x2 window extreme of z
+                if tc and (role == "s" or not pooled):
+                    w[f"{role}.{mod}.z{li}"] = e(N, co // 8, ho, ho, 8, dtype=torch.float16)   # act8 layout, fp16: never an MMA operand
+                elif not tc:
+                    w[f"{role}.{mod}.z{li}"] = e(N, co, ho, ho)
+                if next_tc:
+                    w[f"{role}.{mod}.p8{li}"] = e(N, co // 8, ho // 2, ho // 2, 8, dtype=BF)
+                if not next_tc or not tc:
+                    w[f"{role}.{mod}.p{li}"] = e(N, co, ho // 2, ho // 2)
+                w[f"{role}.{mod}.stats{li}"] = zalloc(nv, co, 2)
+                for nm in ("scale", "shift", "mean", "invstd"):
+                    w[f"{role}.{mod}.{nm}{li}"] = e(nv, co)
+                if role != "s":
+                    continue
+                w[f"s.{mod}.sums{li}"] = zalloc(nv, co, 2)
+                if tc:
+                    sc["wg"] = max(sc["wg"], ops.conv_tc_wgrad_work_floats(N, ci, co, hw, hw, k, pad))
+                    if ci == 1:
+                        # fused apply + weight gradient: this layer's dz never exists in HBM
+                        sc["wg"] = max(sc["wg"], ops.conv_tc_wgrad_l0_fused_work_floats(N, B, co, hw, hw, k, pad))
+                    else:
+                        sc["z8"] = max(sc["z8"], N * co * ho * ho)
+                else:
+                    sc["wg"] = max(sc["wg"], ops.conv_bwd_weight_work_floats(N, ci, co, hw, hw, k, pad))
+                    sc["z"] = max(sc["z"], N * co * ho * ho)
+                sc["p"] = max(sc["p"], N * co * (ho // 2) * (ho // 2), N * ci * hw * hw if li > 0 else 0)
+            if role == "s" and layers:
+                w[f"{mod}.dz"] = e(max(sc["z"], 4))
+                w[f"{mod}.dz8"] = e(max(sc["z8"], 8), dtype=BF)
+                w[f"{mod}.dz8b"] = e(max(sc["z8"], 8), dtype=BF)      # second buffer: the weight gradient of layer l overlaps layer l-1
+                w[f"{mod}.dbsum"] = zalloc(8, 256)
+                w[f"{mod}.dp_a"], w[f"{mod}.dp_b"] = e(sc["p"]), e(sc["p"])
+                w[f"{mod}.wg_work"] = e(max(sc["wg"], 4))
+                w[f"{mod}.wg_work_b"] = e(max(sc["wg"], 4))
 
     def _uni_workspace(self, w, role, N, e, with_feat=True):
         """Unimodal kinds: the stack's top features "top" [N, W] and the outputs of the linears after it (`feat` [N, O] last).  An
@@ -870,8 +836,6 @@ class DinoStepEngine:
             tc = self.tc[mod][li]
             next_tc = li + 1 < len(layers) and self.tc[mod][li + 1]
             pooled = tc and self.pool["s" if role == "s" else "t"][mod][li]
-            if "zarena" not in w:
-                stats.zero_()
             wrole = role if role in ("s", "t") else self._eval_wrole      # the evaluation role "e" borrows a role's weight images
             if tc:
                 xin = cur
@@ -910,8 +874,6 @@ class DinoStepEngine:
         M = x.shape[0]
         ops.linear_fwd(x, P[prefix + "mlp.0.weight"], P[prefix + "mlp.0.bias"], hh, tc=self.lin_tc)
         st = w[f"{role}.{tag}hstats"]
-        if "zarena" not in w:
-            st.zero_()
         ops.colstats(hh, st)
         ops.bn_finalize(st, P[prefix + "mlp.1.weight"], P[prefix + "mlp.1.bias"], bn.running_mean, bn.running_var, bn.num_batches_tracked,
                         w[f"{role}.{tag}hscale"], w[f"{role}.{tag}hshift"], w[f"{role}.{tag}hmean"], w[f"{role}.{tag}hinvstd"], 1, M)
@@ -935,8 +897,6 @@ class DinoStepEngine:
         self._lin_wgrad(d_out, g, G[prefix + "mlp.4.weight"], G[prefix + "mlp.4.bias"])
         ops.linear_bwd_data(d_out, S[prefix + "mlp.4.weight"], d_g, tc=self.lin_tc)
         sums = w[f"{role}.{tag}hsums"]
-        if "zarena" not in w:
-            sums.zero_()
         sc, sh, mu, inv = (w[f"{role}.{tag}h{n}"] for n in ("scale", "shift", "mean", "invstd"))
         ops.bn1d_gelu_drop_bwd_reduce(hh, d_g, sc, sh, mu, inv, mask, drop_p, sums)
         ops.bn1d_gelu_drop_bwd_apply(hh, d_g, sc, sh, mu, inv, mask, drop_p, sums, d_hh)
@@ -998,8 +958,6 @@ class DinoStepEngine:
         S, G = self.S, self.G
         d_p = d_top
         BF = torch.bfloat16
-        if any(self.tc[mod]) and "zarena" not in w:
-            w[f"{mod}.dbsum"].zero_()
         # weight gradients (UMMA-issue bound, little HBM traffic) run on their own stream beside the data gradient and the next
         # layer's HBM-bound BatchNorm kernels; dz and the wgrad scratch are double-buffered, an event guards their reuse
         main = torch.cuda.current_stream()
@@ -1011,8 +969,6 @@ class DinoStepEngine:
             tc = self.tc[mod][li]
             z = w[f"s.{mod}.z{li}"]
             sums = w[f"s.{mod}.sums{li}"]
-            if "zarena" not in w:
-                sums.zero_()
             sc, sh, mu, inv = (w[f"s.{mod}.{n}{li}"] for n in ("scale", "shift", "mean", "invstd"))
             if tc:
                 if d_p.dtype != BF:
@@ -1094,34 +1050,18 @@ class DinoStepEngine:
         key = ("eval", B)
         if key in self._ws:
             return self._ws[key]
-        dev, BF = self.device, torch.bfloat16
+        dev = self.device
         w = {"B": B}
 
         def e(*shape, dtype=F32):
             return torch.empty(*shape, dtype=dtype, device=dev)
 
+        w["zarena"], zalloc = _zero_arena(1 << 12, dev)
         if self.img_layers:
             w["x_img"] = e(B, 1, 28, 28)
         if self.aud_layers:
             w["x_aud"] = e(B, 1, 112, 112)
-        for mod, layers in (("img", self.img_layers), ("aud", self.aud_layers)):
-            for li, (conv, bn, ci, co, hw, k, pad) in enumerate(layers):
-                ho = hw + 2 * pad - k + 1
-                tc = self.tc[mod][li]
-                next_tc = li + 1 < len(layers) and self.tc[mod][li + 1]
-                if tc and ci == 1:
-                    w[f"{mod}.xs8"] = e(B, hw, ops.quad8_width(hw, pad), 8, dtype=BF)
-                if tc and self.pool["t"][mod][li]:
-                    w[f"e.{mod}.e{li}"] = e(B, co // 8, ho // 2, ho // 2, 8, dtype=torch.float16)
-                else:
-                    w[f"e.{mod}.z{li}"] = e(B, co // 8, ho, ho, 8, dtype=torch.float16) if tc else e(B, co, ho, ho)
-                if next_tc:
-                    w[f"e.{mod}.p8{li}"] = e(B, co // 8, ho // 2, ho // 2, 8, dtype=BF)
-                if not next_tc or not tc:
-                    w[f"e.{mod}.p{li}"] = e(B, co, ho // 2, ho // 2)
-                w[f"e.{mod}.stats{li}"] = torch.zeros(1, co, 2, dtype=torch.float64, device=dev)
-                for nm in ("scale", "shift", "mean", "invstd"):
-                    w[f"e.{mod}.{nm}{li}"] = e(1, co)
+        self._stack_buffers(w, "e", B, B, e, zalloc)
         E, O = self.E, self.O
         if self.multi:
             self._mix_workspace(w, "e", B, B, B, e)
@@ -1150,7 +1090,6 @@ class DinoStepEngine:
             bns[k] = c
         return {"bns": bns, "step": 0, "teacher": teacher}
 
-    @_main_chain
     @torch.no_grad()
     def encode_features(self, images, audios=None, train=False, teacher=False, probe=None, step_dev=None):
         """Encoder features [B, O] of an UN-augmented batch (images [B,28,28] fp32 in [0,1] or uint8, audios [B,112,112] fp32 in
@@ -1193,12 +1132,12 @@ class DinoStepEngine:
             else:
                 ops.dropout_mask(fmask, self.fusion_dropout, self.seed + 17, (self.rng_step + (probe["step"] if probe is not None else 0)) * 4 + 3)
         self._eval_wrole = "t" if teacher else "s"
+        w["zarena"].zero_()                             # the BatchNorm statistics of every layer
         return self._encode(w, "e", P, bns, xi, xa, B, B, B, fmask, train=train)
 
     # ------------------------------------------------------------------------------------------------------
     # the step
     # ------------------------------------------------------------------------------------------------------
-    @_main_chain
     def forward_pass(self, x_img, x_aud, masks=None, raw=None):
         """Student (all views [+ the un-augmented pass in the non-default modes]) and teacher (global views) forward
         through encoders and heads.  Returns the workspace dict; outputs: w['s.proj'] [V*B,P], w['t.proj'] [Vg*B,P]
@@ -1277,7 +1216,6 @@ class DinoStepEngine:
         w["loss"].zero_()
         return w
 
-    @_main_chain
     def dino_loss_pass(self, w):
         """Fused DINO loss forward+backward (fills w['d.proj'], loss[0]) and the centre EMA (all-reduced when data parallel)."""
         V, Vg, P, B = self.V, self.Vg, self.P, w["B"]
@@ -1308,7 +1246,6 @@ class DinoStepEngine:
             torch.cuda.current_stream().wait_event(self._center_ready)
             self._center_ready = None
 
-    @_main_chain
     def aux_loss_pass(self, w, labels=None):
         """MSE / InfoNCE / CE on the mode heads' outputs, forward+backward fused (fills w['aux_*.d.out'], loss[1])."""
         loss = w["loss"]
@@ -1323,7 +1260,6 @@ class DinoStepEngine:
         elif self.mode == "mse":
             ops.mse_align_fwd_bwd(oi, oa, w["aux_image.d.out"], w["aux_audio.d.out"], loss[1:2], grad_scale=self.alpha, work=w["loss_work"])
 
-    @_main_chain
     def backward_pass(self, w, d_proj=None, d_aux=None):
         """Backward from the gradient w.r.t. the student projections (default: the fused loss's own w['d.proj']) and, in the
         non-default modes, w.r.t. the two mode-head outputs (default: w['aux_*.d.out']).  Fills self.grad."""
@@ -1366,8 +1302,6 @@ class DinoStepEngine:
                     p_last = w[f"s.{mod}.p{len(layers) - 1}"]
                     x_lin = w[f"s.{mod}.gap"] if pool else p_last.view(Ns, nflat)
                     self._lin_wgrad(d_catr[:, sl], x_lin, G[lin + ".weight"], G[lin + ".bias"])
-                    if mod == "aud" and self.world > 1 and self.overlap_grad_exchange:
-                        self._exchange_late_gradients()
                     if pool:
                         ops.linear_bwd_data(d_catr[:, sl], S[lin + ".weight"], w[f"d.{mod}.gap"], tc=self.lin_tc)
                         d_p = w[f"{mod}.dp_a"][:p_last.numel()].view_as(p_last)
@@ -1398,20 +1332,6 @@ class DinoStepEngine:
         if self.world > 1:
             self.allreduce_gradients()
 
-    def _exchange_late_gradients(self):
-        """The gradients of [audio encoder linear | fusion MLP | projection head] (+ the mode heads) are complete once the linear
-        weight gradients issued so far are: all-reduce them on the communication stream while the conv stacks run backward."""
-        main, cs = torch.cuda.current_stream(), self._comm_stream
-        cs.wait_stream(main)
-        if self._lin_wg_pending:
-            cs.wait_stream(self._lin_wg_stream)
-        with torch.cuda.stream(cs):
-            self.comm.allreduce_grads_(self.grad[self._bucket_split:self.n_trainable_prefix], cs.cuda_stream)
-            if self.aux_range is not None:
-                self.comm.allreduce_grads_(self.grad[self.aux_range[0]:self.aux_range[1]], cs.cuda_stream)
-        self._comm_pending = "late"
-
-    @_main_chain
     def forward_backward(self, x_img, x_aud, masks=None, raw=None, labels=None):
         """Student + teacher forward, losses, centre EMA and the full backward for already-augmented views.
 
@@ -1431,26 +1351,21 @@ class DinoStepEngine:
         return loss
 
     def allreduce_gradients(self):
-        """Data parallel exchange of the gradient arena through the C ABI (NCCL): the slices that were not exchanged during the
-        backward pass, on the communication stream; Adam joins that stream.  The 1/world average is folded into Adam's grad_scale."""
+        """Data parallel exchange of the gradient arena through the C ABI (NCCL), once the backward pass has joined its streams: on
+        the communication stream, where it overlaps the teacher EMA; Adam joins that stream.  The 1/world average is folded into
+        Adam's grad_scale.  (Exchanging the early-complete slices beside the conv stacks' backward measured slower: DESIGN.md.)"""
         main, cs = torch.cuda.current_stream(), self._comm_stream
         cs.wait_stream(main)
         with torch.cuda.stream(cs):
-            if self._comm_pending == "late":
-                if self._bucket_split > 0:
-                    self.comm.allreduce_grads_(self.grad[:self._bucket_split], cs.cuda_stream)
-            else:
-                for lo, hi in self.grad_plan.ranges:
-                    self.comm.allreduce_grads_(self.grad[lo:hi], cs.cuda_stream)
+            for lo, hi in self.grad_plan.ranges:
+                self.comm.allreduce_grads_(self.grad[lo:hi], cs.cuda_stream)
         self._comm_pending = True
         self._grad_scale = 1.0 / self.world
 
-    @_main_chain
     def update_teacher(self):
         """Teacher EMA over the whole common arena prefix: one kernel (models/dino.py:635-646)."""
         ops.ema_flat(self.teacher.flat[:self.n_ema], self.student.flat[:self.n_ema], self.momentum)
 
-    @_main_chain
     def optimizer_step(self, grad_scale=None):
         """Adam (lr, weight_decay; models/dino.py:953-962) over the parameters that received gradients."""
         self.step_count += 1
@@ -1491,7 +1406,6 @@ class DinoStepEngine:
         if self._ctr is not None:
             self._ctr[1:2].fill_(self.step_count)
 
-    @_main_chain
     def train_step_views(self, x_img, x_aud, masks=None, raw=None, labels=None):
         """Reference step order on given views: forward/loss/backward, EMA (before the optimizer, dino.py:871), Adam."""
         loss = self.forward_backward(x_img, x_aud, masks=masks, raw=raw, labels=labels)
@@ -1503,7 +1417,6 @@ class DinoStepEngine:
             ops.counters_advance(self._ctr)
         return loss
 
-    @_main_chain
     def train_step(self, images, audios=None, labels=None):
         """Whole step from a raw device batch: images [B,28,28] fp32 in [0,1] or uint8; audios [B,112,112] uint8 (or fp32);
         labels int64 [B] (semi_supervised).  Returns the device loss tensor [4] (dino, aux, cosine, total)."""
