@@ -453,22 +453,38 @@ class FeatureExtractor(nn.Module):
     """Frozen student-encoder features of un-augmented batches.  The reference deep-copies the encoder; here the weights are the
     live student's (identical while nothing trains in between) and the part of the copy that DOES change during a probe -- the
     BatchNorm running statistics, which adapt in train() mode and are read in eval() mode -- is a per-extractor copy held by the
-    engine (DinoStepEngine.begin_probe).  train()/eval() select batch / running statistics exactly like the copy's mode would."""
+    engine (DinoStepEngine.begin_probe).  train()/eval() select batch / running statistics exactly like the copy's mode would.
+
+    is_dino_based=False: a stand-alone contrastive container (InfoNCEModel or MultiModalSimCLRModel; a Lightning module passes its
+    `.model`).  Its features are cat([image_encoder(images), audio_encoder(spectrograms)], 1), so output_dim = 2 * the container's
+    output_dim; the projection heads are not part of them.  The BatchNorm rules are the same, through ContrastiveStepEngine.begin_probe.
+    The reference's body of this branch is not in this tree: these semantics are stated, not pinned (DESIGN.md section 4.12)."""
 
     def __init__(self, pretrained_model, is_dino_based=True):
         super().__init__()
-        if not is_dino_based or not hasattr(pretrained_model, "_b200"):
-            raise NotImplementedError("only DINO models with a compiled B200 step have a CUDA feature path")
-        self._dino = [pretrained_model]                      # not registered: the encoder stays owned by the DINO model
-        self.is_unimodal = hasattr(pretrained_model.student, "modality")
-        self.modality = getattr(pretrained_model.student, "modality", None)
-        self.output_dim = pretrained_model.student.output_dim
+        if is_dino_based:
+            if not hasattr(pretrained_model, "_b200"):
+                raise NotImplementedError("only DINO models with a compiled B200 step have a CUDA feature path")
+            self.is_unimodal = hasattr(pretrained_model.student, "modality")
+            self.modality = getattr(pretrained_model.student, "modality", None)
+            self.output_dim = pretrained_model.student.output_dim
+        else:
+            if B.contrastive_binding(pretrained_model) is None:
+                raise NotImplementedError("is_dino_based=False takes an InfoNCEModel or MultiModalSimCLRModel container")
+            self.is_unimodal, self.modality = False, None
+            self.output_dim = 2 * pretrained_model.output_dim
+        self.is_dino_based = is_dino_based
+        self._dino = [pretrained_model]                      # not registered: the encoder stays owned by the pretrained model
         self._probe = None
+
+    def engine(self):
+        """The step engine that computes the features (created and bound on first use)."""
+        m = self._dino[0]
+        return m._b200.ensure(m.center.device) if self.is_dino_based else B.contrastive_binding(m).ensure_eval()
 
     @torch.no_grad()
     def forward(self, images, spectrograms=None):
-        dino = self._dino[0]
-        eng = dino._b200.ensure(dino.center.device)
+        eng = self.engine()
         if self._probe is None:
             self._probe = eng.begin_probe()
         img = aud = None
@@ -482,7 +498,8 @@ class FeatureExtractor(nn.Module):
 
 
 class DownstreamClassifier(nn.Module):
-    """Frozen encoder + Linear(output_dim, 128) -> ReLU -> Linear(128, num_classes) (reference models/dino.py:1764-1815)."""
+    """Frozen encoder + Linear(output_dim, 128) -> ReLU -> Linear(128, num_classes) (reference models/dino.py:1764-1815).
+    is_dino_based=False: a contrastive container's encoders, output_dim = 2 * its output_dim (FeatureExtractor)."""
 
     def __init__(self, pretrained_model, num_classes=10, trainable_encoder=False, is_dino_based=True):
         super().__init__()

@@ -17,6 +17,8 @@ from multimodal_ssl_avmnist_b200 import binding as B  # noqa: E402
 
 
 class InfoNCEModel(nn.Module):
+    B200_CONTRASTIVE_KIND = "infonce"          # the ContrastiveStepEngine kind a bare container is bound to
+
     def __init__(self, output_dim=256, projection_dim=256):
         super().__init__()
         self.output_dim, self.projection_dim = output_dim, projection_dim

@@ -9,7 +9,9 @@ Downstream evaluation: `feature_extraction_loop` / `train_knn_classifier` (refer
 the device kNN kernels (SURVEY 8f-3); `train_downstream` (the 10-epoch MLP probe on frozen features) runs on the device probe
 kernels (multimodal_ssl_avmnist_b200/probe.py, DESIGN.md section 4.11); `compute_classification_metrics` reduces a confusion
 matrix accumulated on the device to sklearn's classification_report; `compute_accuracies` is the post-training evaluation of
-the reference's run_dino.py:389 (kNN + MLP probe + metrics)."""
+the reference's run_dino.py:389 (kNN + MLP probe + metrics).  With is_dino_based=False every one of them evaluates a stand-alone
+contrastive container (InfoNCEModel / MultiModalSimCLRModel) instead: its features are its two encoders' outputs side by side
+(models.dino.FeatureExtractor, DESIGN.md section 4.12)."""
 import csv
 import json
 import os
@@ -94,7 +96,8 @@ class B200KNN:
 
 def train_knn_classifier(pretrained_dino, train_dataloader, test_dataloader, n_neighbors=5, device="cuda", is_dino_based=True):
     """kNN accuracy of the frozen student encoder (reference :349-369): features through the CUDA encoder forward, Euclidean
-    k-nearest neighbours + majority vote in CUDA kernels (csrc/knn.cu).  Returns (knn, accuracy in %)."""
+    k-nearest neighbours + majority vote in CUDA kernels (csrc/knn.cu).  is_dino_based=False: the frozen encoders of a contrastive
+    container (InfoNCEModel / MultiModalSimCLRModel), features [N, 2 * output_dim].  Returns (knn, accuracy in %)."""
     from models.dino import FeatureExtractor
     extractor = FeatureExtractor(pretrained_dino, is_dino_based=is_dino_based)
     train_features, train_labels = feature_extraction_loop(device, extractor, train_dataloader)
@@ -114,6 +117,7 @@ def train_downstream(pretrained_model, train_loader, test_loader, num_epochs=10,
     evaluation of test_loader with eval-mode features after every epoch.  Every step runs on the device (probe.ProbeSession).
     Returns (classifier, history): classifier is a DownstreamClassifier holding the trained head, so classifier(images,
     spectrograms) works afterwards; history = {"train_loss", "val_loss", "val_acc" (%)} per epoch, losses per sample.
+    is_dino_based=False: the probe of a contrastive container's frozen encoders (no dropout; head Linear(2 * output_dim, 128)).
     The reference's body of this function is not in this tree: the signature and the semantics follow its call site and
     models/dino.py's DownstreamClassifier, not a pinned implementation."""
     from models.dino import DownstreamClassifier
@@ -133,7 +137,7 @@ def train_downstream(pretrained_model, train_loader, test_loader, num_epochs=10,
         history["val_acc"].append(100.0 * ev["accuracy"])
         print(f"Epoch {epoch + 1}/{num_epochs}: train loss {train_loss:.4f}, val loss {ev['loss']:.4f}, val acc {100.0 * ev['accuracy']:.2f}%")
     session.export_head()
-    classifier.to(pretrained_model.center.device).eval()
+    classifier.to(session.device).eval()
     classifier.b200_probe = session
     return classifier, history
 
@@ -171,15 +175,14 @@ def compute_classification_metrics(classifier, loader, device="cuda", num_classe
     """Accuracy, per-class precision / recall / f1-score / support, macro and weighted averages (sklearn's
     classification_report(output_dict=True, zero_division=0) definitions) and the int64 confusion matrix of a DownstreamClassifier
     on `loader`.  Predictions and the confusion matrix are computed on the device (eval-mode features -> probe kernel); only the
-    [C, C] matrix comes back to the host."""
+    [C, C] matrix comes back to the host.  Works for a DINO-based and a contrastive (is_dino_based=False) classifier alike."""
     from multimodal_ssl_avmnist_b200.probe import ProbeSession
     session = getattr(classifier, "b200_probe", None)
     if session is None or session.C != num_classes:
         fx = classifier.encoder
-        dino = fx._dino[0]
         if fx._probe is None:
-            fx._probe = dino._b200.ensure(dino.center.device).begin_probe()
-        session = ProbeSession(dino, num_classes=num_classes, graph=False, head=classifier.classifier, probe=fx._probe)
+            fx._probe = fx.engine().begin_probe()
+        session = ProbeSession(fx._dino[0], num_classes=num_classes, graph=False, head=classifier.classifier, probe=fx._probe)
     else:
         session.load_head(classifier.classifier)
     return metrics_from_confusion(session.evaluate(loader)["confusion_matrix"])
@@ -188,7 +191,9 @@ def compute_classification_metrics(classifier, loader, device="cuda", num_classe
 def compute_accuracies(pretrained_model, train_loader, test_loader, n_neighbors=5, num_epochs=10, learning_rate=1e-3, device="cuda",
                        num_classes=10, is_dino_based=True):
     """Post-training evaluation of a pretrained DINO model (reference run_dino.py:389): kNN accuracy of the frozen student's
-    features, the MLP probe (train_downstream) and its classification metrics on test_loader.
+    features, the MLP probe (train_downstream) and its classification metrics on test_loader.  is_dino_based=False: the same for a
+    contrastive container (InfoNCEModel / MultiModalSimCLRModel; a Lightning module passes its .model); its parameters, BatchNorm
+    buffers and optimiser state are left untouched.
     Returns {"knn_acc": %, "mlp_acc": %, "metrics": compute_classification_metrics(...)}."""
     _, knn_acc = train_knn_classifier(pretrained_model, train_loader, test_loader, n_neighbors=n_neighbors, device=device,
                                       is_dino_based=is_dino_based)

@@ -370,10 +370,20 @@ class ContrastiveAdam(torch.optim.Optimizer):
 
 class ContrastiveBinding:
     """Adopts the parameters / BatchNorm buffers of an InfoNCEModel or MultiModalSimCLRModel container into a ContrastiveStepEngine
-    (module tensors become views of the engine's arena) and runs the reference's training_step on it."""
+    (module tensors become views of the engine's arena) and runs the reference's training_step on it.  It registers itself on the
+    container (`model._b200_contrastive`), so that the evaluation entry points find the engine from the container alone."""
 
     def __init__(self, model, kind):
         self.model, self.kind, self.engine = model, kind, None
+        model._b200_contrastive = self
+
+    def ensure_eval(self):
+        """The engine for evaluation: on the device of the container's parameters, or the current CUDA device for a container
+        still on the host (whose parameters are then adopted there, as a first training step would)."""
+        if not torch.cuda.is_available():
+            raise ops._lib.B200Error("contrastive evaluation needs a CUDA device: the feature path has no CPU fallback")
+        p = next(self.model.parameters())
+        return self.ensure(p.device if p.is_cuda else torch.device("cuda", torch.cuda.current_device()))
 
     def ensure(self, device):
         from .contrastive import ContrastiveStepEngine
@@ -415,3 +425,13 @@ class ContrastiveBinding:
             p.grad = eng.G["enc." + name] if name.split(".", 1)[0] in live else None
         anchor = next(self.model.parameters())
         return _AppliedLoss.apply(loss[3], anchor)
+
+
+def contrastive_binding(model):
+    """The ContrastiveBinding of an InfoNCEModel / MultiModalSimCLRModel container: the registered one, or a new one whose kind
+    comes from the container's class (`B200_CONTRASTIVE_KIND`).  None for any other object."""
+    b = getattr(model, "_b200_contrastive", None)
+    if b is not None:
+        return b
+    kind = getattr(type(model), "B200_CONTRASTIVE_KIND", None)
+    return None if kind is None else ContrastiveBinding(model, kind)

@@ -12,6 +12,9 @@ parameter, so the branch (encoder + head of one modality) that a SimCLR step did
 The engine reuses DinoStepEngine's building blocks (tensor-core conv stacks with their fused first-layer backward, BatchNorm / pool
 kernels, linear kernels, flat-arena Adam) with its own parameter inventory and schedule; parameters are named as in the reference's
 state_dict (`image_encoder.encoder.0.weight`, `audio_projection_head.mlp.4.bias`, ...).  No CPU fallback.
+
+Evaluation: encode_features / begin_probe give the frozen features cat([image_encoder(x), audio_encoder(x)], 1) on the same
+conv-stack kernels, for the kNN and MLP-probe evaluation (FeatureExtractor(model, is_dino_based=False), probe.ProbeSession).
 """
 import math
 
@@ -127,11 +130,85 @@ class ContrastiveStepEngine(DinoStepEngine):
 
     def _dino_only(self, *a, **k):
         raise ops._lib.B200Error("this entry point belongs to the DINO step engine; the contrastive engine offers forward_backward / "
-                                 "optimizer_step / train_step_views / train_step / capture_train_step / graph_step")
+                                 "optimizer_step / train_step_views / train_step / capture_train_step / graph_step / begin_probe / "
+                                 "encode_features")
 
     # inherited DINO-specific entry points that have no meaning here
-    forward_pass = dino_loss_pass = aux_loss_pass = backward_pass = update_teacher = train_step_host = encode_features = begin_probe = _dino_only
+    forward_pass = dino_loss_pass = aux_loss_pass = backward_pass = update_teacher = train_step_host = _dino_only
     augment = augment_with_params = prefetch_augment = allreduce_gradients = graph_node_counts = _dino_only
+
+    # ------------------------------------------------------------------------------------------------------
+    # evaluation-side encoder forward: frozen features for the kNN and MLP-probe evaluation (DESIGN.md section 4.12)
+    # ------------------------------------------------------------------------------------------------------
+    def _eval_workspace(self, B):
+        key = ("eval", B)
+        if key in self._ws:
+            return self._ws[key]
+        dev = self.device
+
+        def e(*shape, dtype=F32):
+            return torch.empty(*shape, dtype=dtype, device=dev)
+
+        w = {"B": B}
+        w["zarena"], zalloc = _zero_arena(1 << 12, dev)
+        w["x_img"], w["x_aud"] = e(B, 1, 28, 28), e(B, 1, 112, 112)
+        self._stack_buffers(w, "e", B, B, e, zalloc)
+        w["img.gap"], w["img.e14"], w["aud.gap"] = e(B, 128), e(B, 512), e(B, 256)
+        w["feat"] = e(B, 2 * self.O)          # [image_encoder(x) | audio_encoder(x)]
+        self._ws[key] = w
+        return w
+
+    def begin_probe(self):
+        """Start a probe session: a token holding a private copy of the seven conv-stack BatchNorms' running statistics (initialised
+        from the live ones), which train-mode encode_features(probe=token) updates and eval-mode reads.  The live statistics are never
+        touched.  The projection heads' BatchNorms are not part of the features and are not copied."""
+        bns = {}
+        for conv, bn, *_ in IMG_LAYERS + AUD_LAYERS:
+            v = self.bn_s["enc." + bn]
+            c = _BN(v.C, self.device)
+            c.running_mean.copy_(v.running_mean)
+            c.running_var.copy_(v.running_var)
+            c.num_batches_tracked.copy_(v.num_batches_tracked)
+            bns["enc." + bn] = c
+        return {"bns": bns, "step": 0, "teacher": False}
+
+    @torch.no_grad()
+    def encode_features(self, images, audios, train=False, probe=None, step_dev=None):
+        """Frozen features [B, 2*O] = cat([image_encoder(images), audio_encoder(audios)], 1) of an UN-augmented batch (images [B,28,28]
+        or [B,1,28,28], audios [B,112,112] or [B,1,112,112]; fp32 in [0, 1] or uint8).  The projection heads are not applied.
+        train=False: BatchNorm with running statistics (module.eval()); train=True: batch statistics.  probe (a begin_probe() token):
+        the running statistics read / updated are the token's; without one, train-mode updates go to scratch and eval reads the live
+        ones.  step_dev is accepted for probe.ProbeSession's captured step; these encoders have no dropout and do not read it.
+        Returns a view of the per-batch-size workspace, overwritten by the next call with the same B."""
+        if images is None or audios is None:
+            raise ops._lib.B200Error("encode_features: a contrastive container's features need both the image and the spectrogram batch")
+        B = self._batch_size(images, audios)
+        w = self._eval_workspace(B)
+        if probe is not None:
+            bns = probe["bns"]
+        elif train:
+            bns = {"enc." + bn: _BN(co, self.device) for conv, bn, ci, co, *_ in IMG_LAYERS + AUD_LAYERS}
+        else:
+            bns = self.bn_s
+        xi, xa = w["x_img"], w["x_aud"]
+        xi.copy_((images.float() / 255.0 if images.dtype == torch.uint8 else images).reshape(B, 1, 28, 28))
+        xa.copy_((audios.float() / 255.0 if audios.dtype == torch.uint8 else audios).reshape(B, 1, 112, 112))
+        self._prep_tc_weights("s", self.S)
+        for mod, layers, x in (("img", IMG_LAYERS, xi), ("aud", AUD_LAYERS, xa)):
+            if self.tc[mod][0]:
+                ops.pack_quad8(x.view(B, layers[0][4], layers[0][4]), w[f"{mod}.xs8"], layers[0][6])
+        w["packed"] = True
+        self._eval_wrole = "s"
+        w["zarena"].zero_()                             # the BatchNorm statistics of every layer
+        S, O, feat = self.S, self.O, w["feat"]
+        pi = self._conv_stack(w, "e", "img", IMG_LAYERS, xi, B, B, S, bns, train=train)
+        ops.avgpool_fwd(pi, w["img.gap"])
+        ops.linear_fwd(w["img.gap"], S["enc.image_encoder.encoder.14.weight"], S["enc.image_encoder.encoder.14.bias"], w["img.e14"], tc=self.lin_tc)
+        ops.linear_fwd(w["img.e14"], S["enc.image_encoder.projection.0.weight"], S["enc.image_encoder.projection.0.bias"], feat[:, :O], tc=self.lin_tc)
+        pa = self._conv_stack(w, "e", "aud", AUD_LAYERS, xa, B, B, S, bns, train=train)
+        ops.avgpool_fwd(pa, w["aud.gap"])
+        ops.linear_fwd(w["aud.gap"], S["enc.audio_encoder.encoder.18.weight"], S["enc.audio_encoder.encoder.18.bias"], feat[:, O:], tc=self.lin_tc)
+        return feat
 
     # ------------------------------------------------------------------------------------------------------
     def _workspace(self, B):

@@ -1,5 +1,6 @@
-"""Downstream MLP probe on the device: a frozen DINO student's features -> DownstreamClassifier's head Linear(O, 128) -> ReLU ->
-Linear(128, C), trained with CrossEntropyLoss and torch.optim.AdamW semantics (DESIGN.md section 4.11).
+"""Downstream MLP probe on the device: the frozen features of a DINO student or of a contrastive container's two encoders ->
+DownstreamClassifier's head Linear(O, 128) -> ReLU -> Linear(128, C), trained with CrossEntropyLoss and torch.optim.AdamW semantics
+(DESIGN.md sections 4.11 and 4.12).
 
 A training batch is encode_features(train=True, probe=token) -> b200_probe_mlp_fwd_bwd -> b200_adam_bias_dev + b200_adamw_flat_dev ->
 b200_counters_advance, all on the device.  The head's parameters, gradient and AdamW moments live in flat arenas laid out as
@@ -12,6 +13,7 @@ import torch.nn as nn
 
 from . import ops
 from ._lib import B200Error
+from .binding import contrastive_binding
 
 HIDDEN = 128
 
@@ -22,19 +24,28 @@ def make_head(in_dim, num_classes):
 
 
 class ProbeSession:
-    """One probe run on a frozen DINO model (anything with a `_b200` DINO binding: MultiModalDINO / UniModalDINO).
+    """One probe run on a frozen DINO model (anything with a `_b200` DINO binding: MultiModalDINO / UniModalDINO) or a stand-alone
+    contrastive container (InfoNCEModel / MultiModalSimCLRModel, whose features are its two encoders' outputs side by side, O = 2 *
+    its output_dim).
 
     head: the nn.Sequential whose initial weights the arena starts from (a fresh make_head() if None); export_head() writes the
-    trained weights back into it.  probe: a DinoStepEngine.begin_probe() token -- the probe's private copy of the BatchNorm running
+    trained weights back into it.  probe: the engine's begin_probe() token -- the probe's private copy of the BatchNorm running
     statistics (a fresh one if None).  graph=True: the training step of the first batch size seen is captured once and replayed;
     other batch sizes (a ragged last batch) run the same launches eagerly."""
 
     def __init__(self, dino_model, num_classes=10, lr=1e-3, weight_decay=1e-2, graph=True, head=None, probe=None):
-        if not hasattr(dino_model, "_b200"):
-            raise B200Error("ProbeSession needs a DINO model with a compiled B200 step")
-        self.device = dino_model.center.device
-        self.eng = dino_model._b200.ensure(self.device)
-        self.O, self.C = int(dino_model.student.output_dim), int(num_classes)
+        if hasattr(dino_model, "_b200"):
+            self.device = dino_model.center.device
+            self.eng = dino_model._b200.ensure(self.device)
+            self.O = int(dino_model.student.output_dim)
+        else:
+            binding = contrastive_binding(dino_model)
+            if binding is None:
+                raise B200Error("ProbeSession needs a DINO model with a compiled B200 step or a contrastive container")
+            self.eng = binding.ensure_eval()
+            self.device = self.eng.device
+            self.O = 2 * int(dino_model.output_dim)
+        self.C = int(num_classes)
         self.lr, self.weight_decay, self.use_graph = float(lr), float(weight_decay), bool(graph)
         self.head = head if head is not None else make_head(self.O, self.C)
         self.token = probe if probe is not None else self.eng.begin_probe()
