@@ -500,7 +500,8 @@ def test_conv_tc_fused_pool_epilogue_is_bit_identical_to_the_unfused_chain(geom,
 
 
 # data gradients (forward geometry: Cin, Cout, H, K, pad) whose epilogue also produces the BN-backward sums of the layer below
-DGRAD_BNSTAT = [(8, 16, 56, 5, 2), (16, 32, 28, 5, 2), (32, 64, 14, 5, 2), (32, 64, 14, 5, 0), (32, 64, 14, 3, 1)]
+DGRAD_BNSTAT = [(8, 16, 56, 5, 2), (16, 32, 28, 5, 2), (32, 64, 14, 5, 2), (32, 64, 14, 5, 0), (32, 64, 14, 3, 1),
+                (64, 128, 7, 3, 1)]        # the last: image_simple conv3 (CfgS2d data gradient, odd 7x7 planes)
 
 
 @pytest.mark.parametrize("geom", DGRAD_BNSTAT)
